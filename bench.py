@@ -8,6 +8,8 @@ all utterances, length-bucketed (padding semantics of the reference: pad to the 
 Every rank runs the full workload on its own GPU (utterance-sharded path, no collective): weak scaling (`value`).
 
   python bench.py --gpus 1 --steps K --warmup W            our arm (CUDA kernels through the C ABI)
+  python bench.py ... --dump-outputs DIR                   also writes what the last timed step computed (a seeded
+                                                           sample of utterances) as DIR/<name>.npy, to compare builds
   python bench.py --impl reference ...                     reference arm: the reference's own classes
                                                            (baseline/_ref/{aptai,modules}.py on transformers, unmodified)
                                                            on the host CPU cores, length-stratified sample
@@ -152,9 +154,47 @@ def make_model(cfg, dev):
 
 
 def hot_path(model, wav, lens, tg, tl):
-    """One batch through the public API: APTAI.predict = encoder + heads + low-pass + argmax + forced alignment."""
-    r = model.predict(wav, lens, phn_targets=tg, phn_target_lens=tl)
-    return r["tvs_pred"], r["phn_fc_pred"], r["align_paths"]
+    """One batch through the public API: APTAI.predict = encoder + heads + low-pass + argmax + forced alignment.
+    Returns what predict() returns to its caller."""
+    return model.predict(wav, lens, phn_targets=tg, phn_target_lens=tl)
+
+
+# --dump-outputs: predict()'s per-frame outputs and their widths
+DUMP_FRAME_KEYS = {"tvs_pred": 9, "phn_fc_logits": 46, "log_probs": 46, "phn_fc_pred": 1, "align_paths": 1,
+                   "align_scores": 1}
+DUMP_BYTES = 60 * 10 ** 6          # with the .npy headers, under 64 MB in all
+
+
+def dump_outputs(out_dir, cfg, lengths, batches, outs, seed=0):
+    """Writes one step's outputs (`outs[k]` = predict() of batches[k]) as float32 `out_dir/<name>.npy`.
+    The files stay within DUMP_BYTES: utterances are taken in a fixed, seeded order while they fit (the config-5
+    step's outputs are several times larger), on their valid frames only (what lies beyond an utterance's length is
+    padding that no caller reads).  Per-frame arrays are the sampled utterances'
+    frames concatenated in utterance-id order, per-utterance arrays (`utterance_index`, `frames`, `align_status`)
+    follow the same order.  The sample depends only on the workload, so two builds dump the same utterances."""
+    frame_bytes = 4 * sum(DUMP_FRAME_KEYS.values())
+    budget = (DUMP_BYTES - 3 * 4 * len(lengths)) // frame_bytes
+    pick, total = [], 0
+    for i in np.random.Generator(np.random.PCG64(seed)).permutation(len(lengths)):
+        n = cfg.conv_out_length(lengths[i])
+        if total + n <= budget:
+            pick.append(int(i))
+            total += n
+    pick.sort()
+    where = {i: (k, j) for k, b in enumerate(batches) for j, i in enumerate(b.indices)}
+    cols = {name: [] for name in (*DUMP_FRAME_KEYS, "align_status")}
+    for i in pick:
+        k, j = where[i]
+        n = cfg.conv_out_length(lengths[i])
+        for name in DUMP_FRAME_KEYS:
+            cols[name].append(outs[k][name][j, :n].float().cpu().numpy())
+        cols["align_status"].append(outs[k]["align_status"][j: j + 1].float().cpu().numpy())
+    os.makedirs(out_dir, exist_ok=True)
+    arrays = {name: np.concatenate(v) for name, v in cols.items()}
+    arrays["utterance_index"] = np.asarray(pick, dtype=np.float32)
+    arrays["frames"] = np.asarray([cfg.conv_out_length(lengths[i]) for i in pick], dtype=np.float32)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, f"{name}.npy"), a.astype(np.float32))
 
 
 class GemmTimer:
@@ -189,6 +229,11 @@ def ensure_reference_copy():
             shutil.copyfile(os.path.join(src, rel), dst)
             manifest[rel] = hashlib.sha256(open(dst, "rb").read()).hexdigest()
         json.dump(manifest, open(os.path.join(REF_DIR, "MANIFEST.json"), "w"), indent=1)
+    return have_reference_copy()
+
+
+def have_reference_copy():
+    """Whether build() left the reference's classes in baseline/_ref/ (the benchmark itself writes nothing there)."""
     return os.path.exists(os.path.join(REF_DIR, "aptai.py"))
 
 
@@ -270,8 +315,9 @@ def stratified_sample(lengths, batches, per_bucket, quantiles):
 def reference_cpu_arm(cfg, lengths, batches, steps, warmup, budget_s):
     """Times the reference's own classes on the host cores.  Returns (audio-s/s, ms per step, description)."""
     torch.set_num_threads(os.cpu_count())
-    if not ensure_reference_copy():
-        raise RuntimeError("baseline/_ref is missing (run __graft_entry__.build() where /root/reference exists)")
+    if not have_reference_copy():
+        raise RuntimeError("baseline/_ref is missing (__graft_entry__.build() copies it from the reference tree "
+                           "named by APTAI_REFERENCE)")
     m = load_reference_aptai(cfg, torch.device("cpu"))
     ref = ReferenceHotPath(m, cfg)
     sample = stratified_sample(lengths, batches, per_bucket=1, quantiles=(0.1, 0.5, 0.9))
@@ -344,10 +390,13 @@ def run_ours(args):
     n_streams = max(1, int(os.environ.get("APTAI_BENCH_STREAMS", "1")))
     side = [torch.cuda.Stream(device=dev) for _ in range(n_streams)] if n_streams > 1 else []
 
-    def step_resident(bs=devb):
+    def step_resident(bs=devb, sink=None):
+        """`sink`: a list that receives each batch's outputs (kept alive only when they are to be dumped)"""
         if not side:
             for (wav, lens, tg, tl) in bs:
-                hot_path(model, wav, lens, tg, tl)
+                r = hot_path(model, wav, lens, tg, tl)
+                if sink is not None:
+                    sink.append(r)
             return
         # independent batches alternate over `n_streams` streams: the tail of one batch's kernel is filled by the
         # other batch's next one, and HBM-bound kernels of one overlap tensor-bound kernels of the other
@@ -356,7 +405,9 @@ def run_ours(args):
             st.wait_stream(cur)
         for i, (wav, lens, tg, tl) in enumerate(bs):
             with torch.cuda.stream(side[i % n_streams]):
-                hot_path(model, wav, lens, tg, tl)
+                r = hot_path(model, wav, lens, tg, tl)
+            if sink is not None:
+                sink.append(r)
         for st in side:
             cur.wait_stream(st)
 
@@ -383,9 +434,9 @@ def run_ours(args):
             main.wait_event(ev)
             for x in (w, l, g, t):
                 x.record_stream(main)
-            tv, pred, paths = hot_path(model, w, l, g, t)
-            sink.append((tv.to("cpu", non_blocking=True), pred.to("cpu", non_blocking=True),
-                         paths.to("cpu", non_blocking=True)))
+            r = hot_path(model, w, l, g, t)
+            sink.append((r["tvs_pred"].to("cpu", non_blocking=True), r["phn_fc_pred"].to("cpu", non_blocking=True),
+                         r["align_paths"].to("cpu", non_blocking=True)))
 
     def barrier():
         if world > 1:
@@ -416,13 +467,23 @@ def run_ours(args):
     clocks.start()
     timer = GemmTimer()
     ops.set_gemm_hook(timer.hook)
-    ms = timed(step_resident, args.steps)
+    last = [] if args.dump_outputs and rank == 0 else None
+
+    def step_timed():
+        if last is not None:
+            last.clear()                             # keep the outputs of the last timed step only
+        step_resident(sink=last)
+
+    ms = timed(step_timed, args.steps)
     ops.set_gemm_hook(None)
     clk = clocks.stop()
     launches = lib.launch_count() - launches0
     gemm_ms = timer.total_ms()
     gemm_launches = len(timer.ev)
     timer.ev.clear()
+    if last is not None:
+        dump_outputs(args.dump_outputs, cfg, lengths, batches, last)
+        last.clear()
     # end-to-end: pinned host -> device copies and device -> host results inside the timed region
     sink = []
     step_e2e(sink)
@@ -596,7 +657,7 @@ def accuracy_mode_leg(model, cfg, lengths, batches, devb, dev):
 def library_baseline_leg(cfg, lengths, batches, dev, ours):
     """The existing Blackwell library path: the reference's classes, torch eager + bf16 autocast (cuBLAS / cuDNN / SDPA)
     on the same GPU, on a stratified third of the same batches; our arm timed on exactly those batches beside it."""
-    if not ensure_reference_copy():
+    if not have_reference_copy():
         return {"unavailable": "baseline/_ref missing"}
     pick = list(range(1, len(batches), 6))
     hs = [synth_batch_host(lengths, batches[k], 1000 * 0 + k, pin=False) for k in pick]
@@ -842,7 +903,12 @@ def main():
     ap.add_argument("--no-train", action="store_true")
     ap.add_argument("--no-accuracy", action="store_true")
     ap.add_argument("--no-library-baseline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last one computed as DIR/<name>.npy (rank 0; float32, "
+                         "valid frames of a fixed, seeded sample of utterances)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.impl == "reference":
         run_reference(args)
     else:

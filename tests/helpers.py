@@ -34,6 +34,25 @@ def golden2():
     return _G2["g"]
 
 
+R4_FRAMES = [399, 352, 299, 221]
+
+
+def r4_targets(T=399):
+    """Phoneme / TV targets of golden_v2's ragged batch R4: int64 [4,T] and fp32 [4,T,9] (-100 beyond each length)."""
+    rng = np.random.Generator(np.random.PCG64(31))
+    phn = np.zeros((4, T), dtype=np.int64)
+    tvt = np.full((4, T, 9), -100.0, dtype=np.float32)
+    for b, n in enumerate(R4_FRAMES):
+        phn[b, :n] = rng.integers(1, 46, size=n)
+        tvt[b, :n] = rng.standard_normal((n, 9), dtype=np.float32)
+    return phn, tvt
+
+
+def f8_tv_targets():
+    """TV targets of golden_v2's Force_APTAI case F8: fp32 [1,399,9]."""
+    return np.random.Generator(np.random.PCG64(51)).standard_normal((1, 399, 9), dtype=np.float32)
+
+
 def cfg_large(**kw):
     return W2V2Config.large(**{**NO_REG, **kw})
 

@@ -220,6 +220,45 @@ def test_aptai_and_pr_parameter_counts_match_reference():
     assert n_backbone + 1024 * 46 + 46 + 51 == 315485921          # what Force_APTAI freezes (row a8)
 
 
+def test_bench_dump_outputs_sample_and_layout(tmp_path, monkeypatch):
+    """bench.py --dump-outputs: float32 files within the byte budget, valid frames of the sampled utterances laid out
+    in utterance order, and the same sample on every run of the same workload."""
+    import numpy as np
+    import bench
+    cfg = cfg_large()
+    lengths, batches = bench.build_workload(cfg, 64, seed=0, max_rows=4096)
+    g = torch.Generator().manual_seed(0)
+    outs = []
+    for b in batches:
+        B, T = len(b.indices), b.frames
+        outs.append({"tvs_pred": torch.randn(B, T, 9, generator=g), "phn_fc_logits": torch.randn(B, T, 46, generator=g),
+                     "log_probs": torch.randn(B, T, 46, generator=g), "phn_fc_pred": torch.randint(0, 46, (B, T)),
+                     "align_paths": torch.randint(-1, 46, (B, T), dtype=torch.int32),
+                     "align_scores": torch.randn(B, T, generator=g), "align_status": torch.zeros(B, dtype=torch.int32)})
+    budget = 2 * 2 ** 20                             # far below the workload's outputs: forces a sample
+    monkeypatch.setattr(bench, "DUMP_BYTES", budget)
+    bench.dump_outputs(str(tmp_path / "a"), cfg, lengths, batches, outs)
+    bench.dump_outputs(str(tmp_path / "b"), cfg, lengths, batches, outs)
+    names = sorted(p.name for p in (tmp_path / "a").iterdir())
+    assert names == sorted(f"{k}.npy" for k in (*bench.DUMP_FRAME_KEYS, "align_status", "utterance_index", "frames"))
+    d = {n[:-4]: np.load(tmp_path / "a" / n) for n in names}
+    assert all(a.dtype == np.float32 for a in d.values())
+    assert sum(a.nbytes for a in d.values()) <= budget
+    for n in names:
+        assert np.array_equal(d[n[:-4]], np.load(tmp_path / "b" / n))
+    idx, fr = d["utterance_index"].astype(int), d["frames"].astype(int)
+    assert 0 < len(idx) < len(lengths) and list(idx) == sorted(set(idx))
+    assert len(d["tvs_pred"]) == fr.sum() and d["phn_fc_logits"].shape == (fr.sum(), 46)
+    where = {i: (k, j) for k, b in enumerate(batches) for j, i in enumerate(b.indices)}
+    off = 0
+    for i, n in zip(idx, fr):
+        k, j = where[i]
+        assert n == cfg.conv_out_length(lengths[i])
+        for name in bench.DUMP_FRAME_KEYS:
+            assert np.array_equal(d[name][off: off + n], outs[k][name][j, :n].float().numpy()), (name, i)
+        off += n
+
+
 def test_precision_modes_are_validated_on_the_host():
     """set_precision accepts the three documented modes on every drop-in module's backbone and refuses anything else
     (no kernels run: host logic only)."""

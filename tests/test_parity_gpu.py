@@ -24,7 +24,8 @@ import torch
 
 pytestmark = pytest.mark.gpu
 
-from helpers import ROOT, TV, VOCAB, backbone_sd, cfg_large, force_tail_state, golden2, pearson
+from helpers import (R4_FRAMES, ROOT, TV, VOCAB, backbone_sd, cfg_large, f8_tv_targets, force_tail_state, golden2,
+                     pearson, r4_targets)
 from aptai_b200 import APTAI, Force_APTAI, Wav2Vec2_PR
 from aptai_b200.backbone import register_in_memory_checkpoint
 from oracle import weights as W
@@ -102,10 +103,9 @@ def test_aptai_single_utterance_8s_20s(aptai_large, mode, tag, L, seed):
 @pytest.mark.parametrize("mode", MODES)
 def test_aptai_forward_ragged_batch(aptai_large, cuda, mode):
     g = golden2()
-    lens, flen = [128000, 113000, 96000, 71000], [399, 352, 299, 221]
+    lens, flen = [128000, 113000, 96000, 71000], R4_FRAMES
     wav = W.waveforms(4, 128000, lens, seed=6234).to(cuda)
-    tvt = torch.from_numpy(g["r4_tvt"]).to(cuda)
-    phn = torch.from_numpy(g["r4_phn"].astype(np.int64)).to(cuda)
+    phn, tvt = (torch.from_numpy(a).to(cuda) for a in r4_targets())
     aptai_large.set_precision(mode)
     try:
         out = aptai_large(0, wav, torch.tensor(lens, device=cuda), phn, *[tvt[:, :, i].contiguous() for i in range(9)])
@@ -191,7 +191,7 @@ def test_force_aptai_8s(cuda, mode):
     tvs = np.stack([np.asarray(out["tvs_pred"][k], dtype=np.float32) for k in TV], -1)
     d = float(np.abs(tvs - g["f8_tvs"]).max())
     fp_agree = float((np.asarray(out["pred_frame_phns"], dtype=np.int64) == g["f8_frame_phns"]).mean())
-    tvt = torch.from_numpy(g["f8_tvt"]).to(cuda)
+    tvt = torch.from_numpy(f8_tv_targets()).to(cuda)
     res = fa(0, wav.to(cuda), torch.tensor([128000], device=cuda), None, None,
              *[tvt[:, :, i].contiguous() for i in range(9)], phn_seqs=[known])
     losses = np.asarray([float(res["loss"]), float(res["tv_loss"]), float(res["align_loss"])])
