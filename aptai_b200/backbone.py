@@ -427,9 +427,9 @@ class Wav2Vec2Backbone(nn.Module):
             # streaming kernel (the backward recomputes statistics and activations from z_i; conv 0 from the waveform)
             y, ws0 = ops.conv0(wav, P.conv0_w, P.conv_b[0], P.conv_ln_w[0], P.conv_ln_b[0], norm, out_dtype=BF16,
                                return_ws=True)
-            conv_sv = SimpleNamespace(wav=wav, ys=[y], zs=[None], affine=None)
-            if norm == 2:        # GroupNorm: per-(utterance, channel) scale / shift computed by the forward kernel
-                conv_sv.affine = ws0[B * 130: B * 130 + B * 1024]
+            conv_sv = SimpleNamespace(wav=wav, ys=[y], zs=[None], gn_saved=None)
+            if norm == 2:        # GroupNorm: per-(utterance, channel) scale / shift and statistics of the forward kernel
+                conv_sv.gn_saved = ops.conv0_groupnorm_saved(ws0, B)
             for i in range(1, len(cfg.conv_kernel)):
                 if norm == 1:
                     z = ops.conv_igemm(y, P.conv_w_bf16[i], P.conv_b[i], cfg.conv_kernel[i], cfg.conv_stride[i], act=0)
@@ -744,8 +744,7 @@ class Wav2Vec2Backbone(nn.Module):
             dz0 = ops.ln_gelu_bwd(dy, T0, pitch, B, P.conv_ln_w[0], P.conv_ln_b[0], 1e-5, G(name + "layer_norm.weight"),
                                   G(name + "layer_norm.bias"), wav=cs.wav, w0t=TP.conv0_wt, bias0=P.conv_b[0])
         else:
-            dz0, sums = ops.conv0_groupnorm_bwd(dy, pitch, cs.wav, T0, P.conv0_w, cs.affine, P.conv_ln_w[0],
-                                                P.conv_ln_b[0])
+            dz0, sums = ops.conv0_groupnorm_bwd(dy, pitch, cs.wav, T0, P.conv0_w, *cs.gn_saved)
             G(name + "layer_norm.bias").add_(sums[:, :, 0].sum(0))
             G(name + "layer_norm.weight").add_(sums[:, :, 1].sum(0))
         if P.conv_b[0] is not None:
@@ -754,7 +753,7 @@ class Wav2Vec2Backbone(nn.Module):
         dw0 = torch.zeros((dz0.shape[1], 64), dtype=F32, device=dz0.device)
         ops.wgrad(dz0, X, dw0)
         G(name + "conv.weight").add_(dw0[:, : cfg.conv_kernel[0]].reshape(-1, 1, cfg.conv_kernel[0]))
-        cs.wav = cs.ys = cs.zs = cs.affine = None
+        cs.wav = cs.ys = cs.zs = cs.gn_saved = None
         release()
 
     # ---- the hot path ----------------------------------------------------------------------------------------

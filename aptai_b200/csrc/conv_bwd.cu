@@ -210,18 +210,20 @@ __global__ void gelu_bwd_rows_kernel(const float* __restrict__ dy, RowMap dy_map
 }
 
 // conv layer 0 with GroupNorm: y = GELU(a * zraw + e), a = gamma * rstd, e = (bias - mean) * a + beta per (utterance,
-// channel) (the forward's `affine` array), zraw recomputed from the waveform.  With g = dy * GELU'(ln):
+// channel) (the forward's `affine` array), zraw recomputed from the waveform.  xhat = (zraw - mean0) * rstd with
+// {mean0, rstd} from the forward's `norm_stats` (mean0 = mean - bias): (ln - beta) / gamma would lose xhat where gamma
+// is 0 and cancel where |gamma| << |beta|.  With g = dy * GELU'(ln):
 //   PASS 1: sums[b][c] = {sum_t g, sum_t g * xhat}         PASS 2: dz = a * (g - S1/T0 - xhat * S2/T0)   (bf16)
 // grid = (frame chunks, B), 256 threads, thread = channels c and c + 256.
 template <int PASS>
 __global__ void __launch_bounds__(256)
 conv0_gn_bwd_kernel(const float* __restrict__ dy, RowMap dy_map, const float* __restrict__ wav, long long wav_ld,
-                    const float* __restrict__ w0, const float* __restrict__ affine, const float* __restrict__ gamma,
-                    const float* __restrict__ beta, int T0, int frames_per_block, float* __restrict__ sums,
+                    const float* __restrict__ w0, const float* __restrict__ affine,
+                    const float* __restrict__ norm_stats, int T0, int frames_per_block, float* __restrict__ sums,
                     __nv_bfloat16* __restrict__ dz) {
   const int b = blockIdx.y;
   const int t_begin = blockIdx.x * frames_per_block, t_end = min(T0, t_begin + frames_per_block);
-  float w[2][10], a[2], e[2], ig[2], bt[2], s1[2] = {0.f, 0.f}, s2[2] = {0.f, 0.f}, m1[2], m2[2];
+  float w[2][10], a[2], e[2], mu[2], rs[2], s1[2] = {0.f, 0.f}, s2[2] = {0.f, 0.f}, m1[2], m2[2];
 #pragma unroll
   for (int h = 0; h < 2; ++h) {
     const int c = threadIdx.x + h * 256;
@@ -229,9 +231,8 @@ conv0_gn_bwd_kernel(const float* __restrict__ dy, RowMap dy_map, const float* __
     for (int k = 0; k < 10; ++k) w[h][k] = __ldg(w0 + c * 10 + k);
     a[h] = affine[(static_cast<long long>(b) * CB_C + c) * 2];
     e[h] = affine[(static_cast<long long>(b) * CB_C + c) * 2 + 1];
-    const float g = __ldg(gamma + c);
-    ig[h] = g != 0.f ? 1.0f / g : 0.f;
-    bt[h] = __ldg(beta + c);
+    mu[h] = norm_stats[(static_cast<long long>(b) * CB_C + c) * 2];
+    rs[h] = norm_stats[(static_cast<long long>(b) * CB_C + c) * 2 + 1];
     if (PASS == 2) {
       m1[h] = sums[(static_cast<long long>(b) * CB_C + c) * 2] / T0;
       m2[h] = sums[(static_cast<long long>(b) * CB_C + c) * 2 + 1] / T0;
@@ -250,7 +251,7 @@ conv0_gn_bwd_kernel(const float* __restrict__ dy, RowMap dy_map, const float* __
 #pragma unroll
       for (int k = 0; k < 10; ++k) zr = fmaf(w[h][k], xs[k], zr);
       const float ln = fmaf(a[h], zr, e[h]);
-      const float xhat = (ln - bt[h]) * ig[h];
+      const float xhat = (zr - mu[h]) * rs[h];
       const float g = __ldg(dy + prow * CB_C + c) * gelu_erf_grad(ln);
       if (PASS == 1) {
         s1[h] += g;
@@ -289,10 +290,10 @@ extern "C" int aptai_gelu_bwd_rows_512(const float* dy, int64_t dy_rows_per_seg,
 }
 
 extern "C" int aptai_conv0_groupnorm_bwd(const float* dy, int64_t dy_seg_pitch, const float* wav, int B, int64_t L,
-                                         int T0, const float* w0, const float* affine, const float* gamma,
-                                         const float* beta, float* sums, void* dz_bf16, void* stream) {
+                                         int T0, const float* w0, const float* affine, const float* norm_stats,
+                                         float* sums, void* dz_bf16, void* stream) {
   if (int rc = check_arch()) return rc;
-  APTAI_REQUIRE(dy && wav && w0 && affine && gamma && beta && sums && dz_bf16, "conv0_groupnorm_bwd: null pointer");
+  APTAI_REQUIRE(dy && wav && w0 && affine && norm_stats && sums && dz_bf16, "conv0_groupnorm_bwd: null pointer");
   APTAI_REQUIRE(B >= 1 && T0 >= 1 && dy_seg_pitch >= T0 && 5LL * (T0 - 1) + 10 <= L, "conv0_groupnorm_bwd: bad shape");
   cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
   cudaError_t e = cudaMemsetAsync(sums, 0, static_cast<size_t>(B) * CB_C * 2 * sizeof(float), st);
@@ -304,9 +305,9 @@ extern "C" int aptai_conv0_groupnorm_bwd(const float* dy, int64_t dy_seg_pitch, 
   const int fpb = 128;
   dim3 grid((T0 + fpb - 1) / fpb, B);
   __nv_bfloat16* dz = reinterpret_cast<__nv_bfloat16*>(dz_bf16);
-  conv0_gn_bwd_kernel<1><<<grid, 256, 0, st>>>(dy, m, wav, L, w0, affine, gamma, beta, T0, fpb, sums, dz);
+  conv0_gn_bwd_kernel<1><<<grid, 256, 0, st>>>(dy, m, wav, L, w0, affine, norm_stats, T0, fpb, sums, dz);
   if (int rc = after_launch("conv0_gn_bwd_sums")) return rc;
-  conv0_gn_bwd_kernel<2><<<grid, 256, 0, st>>>(dy, m, wav, L, w0, affine, gamma, beta, T0, fpb, sums, dz);
+  conv0_gn_bwd_kernel<2><<<grid, 256, 0, st>>>(dy, m, wav, L, w0, affine, norm_stats, T0, fpb, sums, dz);
   return after_launch("conv0_gn_bwd");
 }
 
@@ -327,6 +328,9 @@ extern "C" int aptai_ln_gelu_bwd_512(const float* dy, int64_t dy_rows_per_seg, i
   APTAI_REQUIRE(dy && gamma && beta && dz_bf16 && dgamma && dbeta && rows >= 1, "ln_gelu_bwd: null pointer");
   APTAI_REQUIRE((z_bf16 != nullptr) != (wav != nullptr && w0t != nullptr), "ln_gelu_bwd: give z, or wav + w0t (conv 0)");
   APTAI_REQUIRE(dy_rows_per_seg >= 1 && dy_seg_pitch >= dy_rows_per_seg, "ln_gelu_bwd: bad row map");
+  APTAI_REQUIRE(z_bf16 || 5 * (dy_rows_per_seg - 1) + 10 <= wav_ld,
+                "ln_gelu_bwd: %lld frames need %lld samples per utterance, the waveform has %lld",
+                (long long)dy_rows_per_seg, 5LL * (dy_rows_per_seg - 1) + 10, (long long)wav_ld);
   RowMap m{dy_rows_per_seg, dy_seg_pitch};
   long long blocks = (rows + 7) / 8;
   const long long cap = 8LL * num_sms();

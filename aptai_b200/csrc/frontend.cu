@@ -99,10 +99,13 @@ __global__ void conv0_gn_moments_kernel(const float* __restrict__ wav, long long
   if (threadIdx.x < K0 + NQ) atomicAdd(&mom[b * (K0 + NQ) + threadIdx.x], red[threadIdx.x]);
 }
 
-// GroupNorm pass B: per (utterance, channel) scale/shift so that out = gelu(conv * a + s).
+// GroupNorm pass B: per (utterance, channel) scale/shift so that out = gelu(conv * a + s).  norm_stats (may be NULL)
+// receives {mean of the bias-free conv output, rstd}: the backward's xhat = (conv - mean) * rstd, which it cannot
+// recover from the scale/shift when gamma is 0 or small.
 __global__ void conv0_gn_affine_kernel(const double* __restrict__ mom, const float* __restrict__ w,
                                        const float* __restrict__ bias, const float* __restrict__ gamma,
-                                       const float* __restrict__ beta, int T0, float eps, float* __restrict__ affine) {
+                                       const float* __restrict__ beta, int T0, float eps, float* __restrict__ affine,
+                                       float* __restrict__ norm_stats) {
   const int b = blockIdx.x;
   const int c = threadIdx.x;
   const double* m = mom + b * (K0 + NQ);
@@ -132,6 +135,10 @@ __global__ void conv0_gn_affine_kernel(const double* __restrict__ mom, const flo
   // y = (conv_nobias + conv_bias - mean) * a + beta
   affine[(b * C0 + c) * 2 + 0] = static_cast<float>(a);
   affine[(b * C0 + c) * 2 + 1] = static_cast<float>((conv_bias - mean) * a + beta[c]);
+  if (norm_stats) {
+    norm_stats[(b * C0 + c) * 2 + 0] = static_cast<float>(mean - conv_bias);
+    norm_stats[(b * C0 + c) * 2 + 1] = static_cast<float>(rstd);
+  }
 }
 
 // NORM: 0 none, 1 LayerNorm over channels per frame, 2 GroupNorm affine per (utterance, channel)
@@ -308,7 +315,7 @@ extern "C" int aptai_conv0_accurate(const float* wav, int B, int64_t L, const fl
     if (chunks > 64) chunks = 64;
     conv0_gn_moments_kernel<<<dim3(chunks, B), 256, 0, st>>>(wav, L, T0, mom);
     if (int rc = after_launch("conv0_gn_moments")) return rc;
-    conv0_gn_affine_kernel<<<B, C0, 0, st>>>(mom, w, bias, gamma, beta, T0, eps, affine);
+    conv0_gn_affine_kernel<<<B, C0, 0, st>>>(mom, w, bias, gamma, beta, T0, eps, affine, nullptr);
     if (int rc = after_launch("conv0_gn_affine")) return rc;
     conv0_accurate_kernel<2><<<grid, 256, 0, st>>>(wav, L, T0, w, bias, gamma, beta, affine, eps, out);
   } else if (norm == 1) {
@@ -326,10 +333,10 @@ int conv0_tc_launch(const float* wav, int B, int64_t L, int T0, const float* w, 
 }
 
 // stats_ws layout: [statistics: norm 1 -> 1 KB of closed-form constants; norm 2 -> B*65 doubles of moments +
-// B*512*2 floats of scale/shift; norm 0 -> nothing] then, 256-byte aligned, the 64 KB split weight operand of the
-// tensor-core kernel
+// B*512*2 floats of scale/shift + B*512*2 floats of {mean, rstd}; norm 0 -> nothing] then, 256-byte aligned, the
+// 64 KB split weight operand of the tensor-core kernel
 static size_t conv0_stats_bytes(int B, int norm) {
-  const size_t s = norm == 1 ? 1024 : (norm == 2 ? sizeof(double) * B * (K0 + NQ) + sizeof(float) * B * C0 * 2 : 0);
+  const size_t s = norm == 1 ? 1024 : (norm == 2 ? sizeof(double) * B * (K0 + NQ) + sizeof(float) * B * C0 * 4 : 0);
   return (s + 255) / 256 * 256;
 }
 extern "C" size_t aptai_conv0_workspace_bytes(int B, int norm) { return conv0_stats_bytes(B, norm) + C0 * 64 * 2; }
@@ -355,9 +362,10 @@ extern "C" int aptai_conv0_norm_gelu(const float* wav, int B, int64_t L, const f
     if (!simt) return conv0_tc_launch(wav, B, L, T0, w, bias, gamma, beta, 1, eps, stats_ws, nullptr, ws_b, out, out_fp16, st);
     conv0_kernel<1><<<grid, 256, 0, st>>>(wav, L, T0, w, bias, gamma, beta, stats_ws, nullptr, eps, out, out_fp16);
   } else if (norm == 2) {
-    // stats_ws: [B*65] doubles of moments, then [B*512*2] floats of scale/shift
+    // stats_ws: [B*65] doubles of moments, then [B*512*2] floats of scale/shift, then [B*512*2] floats of {mean, rstd}
     double* mom = reinterpret_cast<double*>(stats_ws);
     float* affine = reinterpret_cast<float*>(mom + static_cast<size_t>(B) * (K0 + NQ));
+    float* norm_stats = affine + static_cast<size_t>(B) * C0 * 2;
     cudaError_t e = cudaMemsetAsync(mom, 0, sizeof(double) * B * (K0 + NQ), st);
     if (e != cudaSuccess) {
       set_error("conv0: memset: %s", cudaGetErrorString(e));
@@ -367,7 +375,7 @@ extern "C" int aptai_conv0_norm_gelu(const float* wav, int B, int64_t L, const f
     if (chunks > 64) chunks = 64;
     conv0_gn_moments_kernel<<<dim3(chunks, B), 256, 0, st>>>(wav, L, T0, mom);
     if (int rc = after_launch("conv0_gn_moments")) return rc;
-    conv0_gn_affine_kernel<<<B, C0, 0, st>>>(mom, w, bias, gamma, beta, T0, eps, affine);
+    conv0_gn_affine_kernel<<<B, C0, 0, st>>>(mom, w, bias, gamma, beta, T0, eps, affine, norm_stats);
     if (int rc = after_launch("conv0_gn_affine")) return rc;
     if (!simt) return conv0_tc_launch(wav, B, L, T0, w, bias, gamma, beta, 2, eps, nullptr, affine, ws_b, out, out_fp16, st);
     conv0_kernel<2><<<grid, 256, 0, st>>>(wav, L, T0, w, bias, gamma, beta, nullptr, affine, eps, out, out_fp16);

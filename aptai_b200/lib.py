@@ -128,7 +128,7 @@ PROTOTYPES = {
                                       c_void_p, c_void_p, c_float, c_void_p, c_void_p, c_void_p, c_void_p]),
     "aptai_gelu_bwd_rows_512": (c_int, [c_void_p, c_i64, c_i64, c_void_p, c_i64, c_void_p, c_void_p]),
     "aptai_conv0_groupnorm_bwd": (c_int, [c_void_p, c_i64, c_void_p, c_int, c_i64, c_int, c_void_p, c_void_p, c_void_p,
-                                          c_void_p, c_void_p, c_void_p, c_void_p]),
+                                          c_void_p, c_void_p, c_void_p]),
     "aptai_conv0_im2col_bf16": (c_int, [c_void_p, c_int, c_i64, c_i64, c_void_p, c_void_p]),
     "aptai_posconv_weightnorm_bwd": (c_int, [c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_void_p,
                                              c_void_p, c_void_p, c_void_p]),

@@ -912,15 +912,24 @@ def gelu_bwd_rows(dy: torch.Tensor, rows_per_seg: int, seg_pitch: int, segs: int
     return dz
 
 
+def conv0_groupnorm_saved(ws: torch.Tensor, B: int):
+    """What the backward of conv layer 0 + GroupNorm needs from `conv0(..., norm=2, return_ws=True)`'s workspace:
+    (affine fp32 [B, 512, 2] = {scale, shift}, norm_stats fp32 [B, 512, 2] = {mean - bias, rstd})."""
+    o = B * 65 * 2                                    # behind the fp64 waveform moments
+    return ws[o: o + B * 1024].view(B, 512, 2), ws[o + B * 1024: o + B * 2048].view(B, 512, 2)
+
+
 def conv0_groupnorm_bwd(dy: torch.Tensor, seg_pitch: int, wav: torch.Tensor, T0: int, w0: torch.Tensor,
-                        affine: torch.Tensor, gamma: torch.Tensor, beta: torch.Tensor):
-    """Backward of conv layer 0 + GroupNorm-over-time + GELU.  Returns (dz0 bf16 [B*T0, 512], sums fp32 [B, 512, 2] =
-    per-utterance {dbeta, dgamma} contributions)."""
-    _req(dy, F32, "dy"); _req(wav, F32, "wav"); _req(affine, F32, "affine")
+                        affine: torch.Tensor, norm_stats: torch.Tensor):
+    """Backward of conv layer 0 + GroupNorm-over-time + GELU (affine, norm_stats: `conv0_groupnorm_saved`).  Returns
+    (dz0 bf16 [B*T0, 512], sums fp32 [B, 512, 2] = per-utterance {dbeta, dgamma} contributions)."""
+    _req(dy, F32, "dy"); _req(wav, F32, "wav"); _req(affine, F32, "affine"); _req(norm_stats, F32, "norm_stats")
     B, L = wav.shape
+    if affine.numel() != B * 1024 or norm_stats.numel() != B * 1024:
+        raise ValueError("conv0_groupnorm_bwd: affine and norm_stats must be [B, 512, 2]")
     sums = torch.empty((B, 512, 2), dtype=F32, device=wav.device)
     dz = torch.empty((B * T0, 512), dtype=BF16, device=wav.device)
     check(_lib.load().aptai_conv0_groupnorm_bwd(dy.data_ptr(), seg_pitch, wav.data_ptr(), B, L, T0, w0.data_ptr(),
-                                                affine.data_ptr(), gamma.data_ptr(), beta.data_ptr(), sums.data_ptr(),
+                                                affine.data_ptr(), norm_stats.data_ptr(), sums.data_ptr(),
                                                 dz.data_ptr(), _stream()), "conv0_groupnorm_bwd")
     return dz, sums

@@ -109,7 +109,8 @@ void aptai_set_traversal(int reverse);
  * channel, statistics over all T0 frames of the padded row (HF:308-323).  norm=0: none (HF:260-272).
  * w is fp32 [512][10]; bias may be NULL.  stats_ws: aptai_conv0_workspace_bytes(B, norm) bytes, 256-byte aligned
  * (normalisation statistics — for norm=2 B*65 doubles of waveform moments followed by the [B][512][2] scale / shift
- * array the backward pass re-uses — then the 64 KB split-bf16 weight operand of the tensor-core kernel).
+ * array and the [B][512][2] {mean - bias, rstd} array the backward pass re-uses — then the 64 KB split-bf16 weight
+ * operand of the tensor-core kernel).
  * flags: bit 0 = the 16-bit output is IEEE fp16 instead of bf16; bit 1 = run the SIMT kernel instead of the
  * tcgen05 one (csrc/conv0_tc.cu: the K = 10 contraction on three-term split bf16 operands, fp32-exact to 2^-24) —
  * for A/B measurements, the results agree to fp32 rounding.
@@ -366,7 +367,8 @@ int aptai_conv_wgrad_bf16(const void* dz, const void* x, int B, int T_out, int T
 /* conv feature encoder, 'layer' norm variant, training path: y = GELU(LayerNorm_512(z)) as a separate streaming kernel
  * (forward), and its backward dz = LN'(dy * GELU'(LN(z))) with dgamma/dbeta accumulated.  dy fp32 with a row map
  * (logical row r of segment s at physical row s*dy_seg_pitch + r).  For conv layer 0 pass z = NULL and wav / w0t
- * ([10][512] transposed weight) / bias0: z is recomputed from the waveform (frame t reads samples 5t .. 5t+9). */
+ * ([10][512] transposed weight) / bias0: z is recomputed from the waveform (frame t reads samples 5t .. 5t+9; wav_ld,
+ * the row pitch, is also the samples per utterance: 5*(dy_rows_per_seg-1)+10 <= wav_ld, else APTAI_ERR_ARG). */
 int aptai_ln_gelu_fwd_512(const void* z_bf16, int64_t rows, const float* gamma, const float* beta, float eps,
                           void* y_bf16, void* stream);
 int aptai_ln_gelu_bwd_512(const float* dy, int64_t dy_rows_per_seg, int64_t dy_seg_pitch, const void* z_bf16,
@@ -374,14 +376,14 @@ int aptai_ln_gelu_bwd_512(const float* dy, int64_t dy_rows_per_seg, int64_t dy_s
                           const float* gamma, const float* beta, float eps, void* dz_bf16, float* dgamma, float* dbeta,
                           void* stream);
 /* 'group' norm variant (base models, HF:308-323).  Layers 1..6 (no norm, no bias): dz = dy * GELU'(z).  Conv layer 0 with
- * GroupNorm over time: affine fp32 [B][512][2] = {gamma*rstd, (bias-mean)*gamma*rstd + beta} as produced by the forward
- * (aptai_conv0_norm_gelu's stats_ws), sums fp32 [B][512][2] receives {sum_t g, sum_t g*xhat} (dbeta / dgamma per
- * utterance), dz bf16 [B*T0][512]. */
+ * GroupNorm over time: affine fp32 [B][512][2] = {gamma*rstd, (bias-mean)*gamma*rstd + beta} and norm_stats fp32
+ * [B][512][2] = {mean - bias, rstd} as produced by the forward (aptai_conv0_norm_gelu's stats_ws), sums fp32
+ * [B][512][2] receives {sum_t g, sum_t g*xhat} (dbeta / dgamma per utterance), dz bf16 [B*T0][512]. */
 int aptai_gelu_bwd_rows_512(const float* dy, int64_t dy_rows_per_seg, int64_t dy_seg_pitch, const void* z_bf16,
                             int64_t rows, void* dz_bf16, void* stream);
 int aptai_conv0_groupnorm_bwd(const float* dy, int64_t dy_seg_pitch, const float* wav, int B, int64_t L, int T0,
-                              const float* w0, const float* affine, const float* gamma, const float* beta, float* sums,
-                              void* dz_bf16, void* stream);
+                              const float* w0, const float* affine, const float* norm_stats, float* sums, void* dz_bf16,
+                              void* stream);
 /* X[b*T0 + t][0..63] = wav[b][5t .. 5t+9], 0-padded, bf16: B operand of conv-0's weight-gradient GEMM */
 int aptai_conv0_im2col_bf16(const float* wav, int B, int64_t L, int64_t T0, void* x_bf16, void* stream);
 /* weight-norm backward (torch parametrizations.weight_norm, dim=2): dg[taps] += , dv[H][cin][taps] += from the
