@@ -514,19 +514,21 @@ def masked_mse_ce(tv_pred, tv_tgt, logits, phn_tgt, return_ws: bool = False):
     return out
 
 
-CTC_MAX_LABELS = 511      # labels per utterance the fused CTC / Viterbi kernels hold (2S+1 states in registers, <= 32 per lane)
+CTC_MAX_LABELS = 4095     # labels per utterance of the CTC / Viterbi kernels (2S+1 states over one CTA, 16 per thread)
 CTC_FAST_LABELS = 127     # up to here (<= 8 states per lane) a padded label tensor is passed as is
 
 
 def _trim_targets(targets: torch.Tensor, target_len: torch.Tensor, what: str) -> torch.Tensor:
     """The kernels' label limit applies to the LONGEST transcript, not to the padded width of the label tensor: a
-    batch padded wider than the limit is narrowed to max(target_len) (one device->host read, only in that case)."""
+    label tensor wider than CTC_FAST_LABELS is narrowed to max(target_len) (one device->host read, only in that
+    case).  The narrowed width selects the kernel: up to 511 labels the state vector lives in one warp's
+    registers, beyond that it spans a CTA."""
     if targets.shape[1] <= CTC_FAST_LABELS:
         return targets
     m = max(1, int(target_len.max()))
     if m > CTC_MAX_LABELS:
         raise ValueError(f"{what}: a transcript of {m} labels exceeds the kernels' limit of {CTC_MAX_LABELS} labels per "
-                         "utterance (INTEGRATION.md, limits); split the utterance")
+                         "utterance (INTEGRATION.md, limits)")
     return targets[:, :m].contiguous()
 
 
@@ -534,7 +536,11 @@ def logsoftmax_ctc(logits: torch.Tensor, targets: torch.Tensor, input_len: torch
                    blank: int = 0, zero_infinity: bool = True, scale: Optional[torch.Tensor] = None,
                    want_log_probs: bool = True, want_grad: bool = False, prepend_blank: bool = False,
                    blank_value: float = 0.0, vocab_len: Optional[torch.Tensor] = None):
-    """Returns dict(nll [B], loss_sum [1], log_probs [T,B,Veff] | None, grad [B,T,V] | None)."""
+    """Returns dict(nll [B], loss_sum [1], log_probs [T,B,Veff] | None, grad [B,T,V] | None).
+
+    Device workspace (`aptai_ctc_workspace_bytes`) is O(B*T*SP): about 2*B*T*SP*4 bytes for alpha and beta, with
+    SP = 32 * (4 | 8 | 16 | 32) up to 511 labels and SP = 512 * ceil((2*S+1) / 512) beyond (S = the longest
+    transcript), e.g. 2.4 GB for B = 16, T = 8999, S = 1000 and 9.4 GB at S = 4095."""
     _req(logits, F32, "logits"); _req(targets, I32, "targets")
     _req(input_len, I32, "input_len"); _req(target_len, I32, "target_len")
     B, T, V = logits.shape

@@ -244,8 +244,15 @@ int aptai_masked_mse_ce(const float* tv_pred, const float* tv_tgt, const float* 
  * targets int32 [B][Smax]; entries at s >= target_len[b] are ignored.  log_probs_tbv (optional) fp32 [T][B][V].
  * nll[b] = -log p(target|input) (0 where infeasible and zero_infinity).  grad (optional) fp32 [B][T][V] is
  * d(sum_b scale[b]*nll[b])/d logits, scale may be NULL (= 1).  Workspace: aptai_ctc_workspace_bytes().
- * Smax <= 511 (the 2 * Smax + 1 DP states are register-resident, 4 / 8 / 16 / 32 per lane; the same limit holds for
- * aptai_ctc_viterbi_f32); aptai_ctc_workspace_bytes() returns 0 beyond it.
+ * Smax <= 4095 labels, for this entry and aptai_ctc_viterbi_f32.  Smax selects the kernel:
+ *   Smax <= 511: one warp holds the 2 * Smax + 1 DP states in registers (4 / 8 / 16 / 32 per lane);
+ *   Smax >  511: the states span one CTA of 32 * ceil((2 * Smax + 1) / 512) threads, 16 per thread (alpha and
+ *                beta CTAs per utterance, frame log-sum-exp and gradient as separate warp-per-frame passes).
+ * Workspace (bytes, each term rounded up to 256, plus 256), SP = padded state count:
+ *   Smax <= 511: 2 * B*T*SP*4 (alpha, beta) + B*T*4 (lse), SP = 32 * (4 | 8 | 16 | 32);
+ *   Smax >  511: 2 * B*T*SP*4 (alpha, beta) + B*T*4 (lse) + 2 * B*T*8 (normalisers) + B*8 (nll)
+ *                + 2 * B*Smax*4 (same-class chains), SP = 512 * ceil((2 * Smax + 1) / 512).
+ * Beyond 4095 labels aptai_ctc_workspace_bytes() returns 0 and the entries return APTAI_ERR_ARG.
  */
 size_t aptai_ctc_workspace_bytes(int B, int T, int Smax);
 int aptai_logsoftmax_ctc(const float* logits, int B, int T, int V, const int32_t* targets, int Smax,
@@ -264,7 +271,11 @@ int aptai_logsoftmax_ctc_ex(const float* logits, int B, int T, int V, int prepen
                             size_t ws_bytes, void* stream);
 
 /* CTC Viterbi forced alignment, bit-exact with torchaudio.functional.forced_align (SURVEY.md Appendix E).
- * log_probs fp32 [B][T][C]; paths int32 [B][T] (frames t >= input_len[b] get -1); scores fp32 [B][T]. */
+ * log_probs fp32 [B][T][C]; paths int32 [B][T] (frames t >= input_len[b] get -1); scores fp32 [B][T].
+ * Smax <= 511: one warp per utterance, back-pointers in shared memory (in the workspace beyond 200 KB);
+ * Smax <= 4095: one CTA per utterance, back-pointers (2 bits per state) always in the workspace,
+ * B*T*128*ceil((2*Smax+1)/512) bytes; beyond 4095 aptai_viterbi_workspace_bytes() returns 0, the entry
+ * APTAI_ERR_ARG. */
 size_t aptai_viterbi_workspace_bytes(int B, int T, int Smax);
 int aptai_ctc_viterbi_f32(const float* log_probs, const int32_t* targets, const int32_t* input_len,
                           const int32_t* target_len, int B, int T, int C, int Smax, int blank, int32_t* paths,
