@@ -113,6 +113,19 @@ def posconv_fold_split(g: torch.Tensor, v: torch.Tensor, cpad: int = 64):
     return hi, lo
 
 
+def pos_conv_add(h: torch.Tensor, w_hi: torch.Tensor, w_lo: torch.Tensor, bias: torch.Tensor, groups: int,
+                 taps: int) -> torch.Tensor:
+    """h fp32 [B,T,H] += gelu(grouped positional conv(h) + bias), in place (HF:329-379, 689-690 | 763-764), as three
+    bf16 products: h_hi.w_hi + h_lo.w_hi + h_hi.w_lo (w_hi / w_lo from posconv_fold_split)."""
+    B, T, H = h.shape
+    hp_hi, hp_lo = cast_pad_split(h, taps // 2)
+    acc = torch.empty_like(h)
+    ops.posconv(hp_hi, w_hi, bias, None, T, H, groups, taps, acc, act=0)
+    ops.posconv(hp_lo, w_hi, None, acc, T, H, groups, taps, acc, act=0)
+    ops.posconv(hp_hi, w_lo, None, acc, T, H, groups, taps, acc, act=0)
+    return gelu_add(acc, h, out=h)
+
+
 def linear3(x3: torch.Tensor, w3: torch.Tensor, bias, **kw):
     """fp32-accurate Linear: x3 = split3(x), w3 = split3(W, weight_layout=True); fp32 output."""
     return ops.linear(x3, w3, bias, want_f32=kw.pop("want_f32", True), want_bf16=False, **kw)[0]
@@ -197,13 +210,8 @@ def encode(m, wav: torch.Tensor, frame_lens: torch.Tensor, *, collect_hidden: bo
     eps, heads = cfg.layer_norm_eps, cfg.num_attention_heads
     _, xn3 = rowop(feats.view(M, -1), P.fp_ln_w, P.fp_ln_b, eps)
     h = linear3(xn3, P.fp_w, P.fp_b, seg_rows=T, seg_valid_rows=frame_lens)
-    taps, groups = cfg.num_conv_pos_embeddings, cfg.num_conv_pos_embedding_groups
-    hp_hi, hp_lo = cast_pad_split(h.view(B, T, H), taps // 2)
-    acc = torch.empty_like(h)
-    ops.posconv(hp_hi, P.pos_w_hi, P.pos_b, None, T, H, groups, taps, acc, act=0)
-    ops.posconv(hp_lo, P.pos_w_hi, None, acc, T, H, groups, taps, acc, act=0)
-    ops.posconv(hp_hi, P.pos_w_lo, None, acc, T, H, groups, taps, acc, act=0)
-    gelu_add(acc, h, out=h)
+    pos_conv_add(h.view(B, T, H), P.pos_w_hi, P.pos_w_lo, P.pos_b, cfg.num_conv_pos_embedding_groups,
+                 cfg.num_conv_pos_embeddings)
     hidden = [] if collect_hidden else None
 
     def attn_ffn(x3, lw, res_attn):

@@ -38,6 +38,7 @@ from . import ops
 from .config import W2V2Config
 
 BF16, F16, F32, I32 = torch.bfloat16, torch.float16, torch.float32, torch.int32
+F32X3_HIDDEN_SIZES = (256, 512, 768, 1024)      # the widths aptai_rowop_split3 is instantiated for
 
 
 # ----------------------------------------------------------------------------------------- parameter containers
@@ -310,6 +311,11 @@ class Wav2Vec2Backbone(nn.Module):
         'f32x3': accuracy mode — every contraction on bf16 hi/lo operand pairs, fp32 elsewhere (inference only)."""
         if precision not in ("bf16", "fp16", "f32x3"):
             raise ValueError(f"aptai_b200: unknown precision {precision!r} ('bf16', 'fp16' or 'f32x3')")
+        if precision == "f32x3" and self.cfg.hidden_size not in F32X3_HIDDEN_SIZES:
+            # the accuracy mode's LayerNorm kernel (aptai_rowop_split3) holds a row in one warp's registers;
+            # head_dim == 64 is already enforced for every mode by cfg.validate_for_kernels()
+            raise ValueError(f"aptai_b200: precision 'f32x3' supports hidden sizes {F32X3_HIDDEN_SIZES}, "
+                             f"not {self.cfg.hidden_size}")
         self.precision = precision       # the fp16 operand copies (0.6 GB for 24x1024) stay cached across mode switches
         return self
 

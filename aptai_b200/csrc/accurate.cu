@@ -263,11 +263,12 @@ extern "C" int aptai_rowop_split3(const float* x, int64_t rows, int cols, const 
   const unsigned grid = static_cast<unsigned>((rows + 7) / 8);
   __nv_bfloat16* o3 = reinterpret_cast<__nv_bfloat16*>(out_split3);
   switch (cols) {
+    case 256: rowop_split3_kernel<8><<<grid, 256, 0, st>>>(x, rows, gamma, beta, eps, norm, gelu, out_f32, o3); break;
     case 512: rowop_split3_kernel<16><<<grid, 256, 0, st>>>(x, rows, gamma, beta, eps, norm, gelu, out_f32, o3); break;
     case 768: rowop_split3_kernel<24><<<grid, 256, 0, st>>>(x, rows, gamma, beta, eps, norm, gelu, out_f32, o3); break;
     case 1024: rowop_split3_kernel<32><<<grid, 256, 0, st>>>(x, rows, gamma, beta, eps, norm, gelu, out_f32, o3); break;
     default:
-      set_error("rowop_split3: cols=%d unsupported (512, 768, 1024)", cols);
+      set_error("rowop_split3: cols=%d unsupported (256, 512, 768, 1024)", cols);
       return APTAI_ERR_ARG;
   }
   return after_launch("rowop_split3");

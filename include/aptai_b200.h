@@ -307,7 +307,7 @@ int aptai_ctc_decode_ref(const float* logits, int B, int T, int V, const int32_t
 int aptai_split3_bf16(const float* x, int64_t rows, int cols, int64_t ld_in, int weight_layout, float scale,
                       void* out_bf16, void* stream);
 /* per row: (LayerNorm, exact two-pass fp32 statistics; HF:431,600-602,639,645,692,792 and the conv LayerNorms
- * HF:288-299) -> (erf-GELU) -> fp32 [rows][cols] and / or split bf16 [rows][3*cols].  cols in {512, 768, 1024}. */
+ * HF:288-299) -> (erf-GELU) -> fp32 [rows][cols] and / or split bf16 [rows][3*cols].  cols in {256, 512, 768, 1024}. */
 int aptai_rowop_split3(const float* x, int64_t rows, int cols, const float* gamma, const float* beta, float eps,
                        int norm, int gelu, float* out_f32, void* out_split3, void* stream);
 /* conv layer 0 + norm + GELU (HF:281-323) in fp32 with split bf16 output [B][T0][3*512]; norm as in

@@ -274,3 +274,17 @@ def test_precision_modes_are_validated_on_the_host():
         with pytest.raises(ValueError):
             m.set_precision(bad)
     assert m.precision == "bf16"
+
+
+@pytest.mark.parametrize("H,heads", [(640, 10), (1280, 20), (128, 2)])
+def test_accuracy_mode_rejects_unsupported_hidden_size_on_the_host(H, heads):
+    """The accuracy mode's row kernel exists for hidden sizes 256 / 512 / 768 / 1024 only: set_precision('f32x3')
+    must refuse any other at the call, naming the supported sizes, and leave the mode unchanged."""
+    from aptai_b200.backbone import Wav2Vec2Backbone
+    cfg = W2V2Config.large(num_hidden_layers=1, hidden_size=H, num_attention_heads=heads, intermediate_size=2 * H,
+                           num_conv_pos_embedding_groups=heads)
+    m = Wav2Vec2Backbone(cfg)
+    with pytest.raises(ValueError, match=r"256, 512, 768, 1024"):
+        m.set_precision("f32x3")
+    assert m.precision == "bf16"
+    assert m.set_precision("fp16").precision == "fp16"
