@@ -16,11 +16,6 @@
 
 namespace aptai {
 
-__device__ __forceinline__ void split_bf16(float x, __nv_bfloat16& hi, __nv_bfloat16& lo) {
-  hi = __float2bfloat16_rn(x);
-  lo = __float2bfloat16_rn(x - __bfloat162float(hi));
-}
-
 // out[r] = [hi | lo | hi] (mode 0, activations) or [hi | hi | lo] (mode 1, weights); x may be strided by ld_in.
 __global__ void split3_kernel(const float* __restrict__ x, long long rows, int cols, long long ld_in, int mode,
                               float scale, __nv_bfloat16* __restrict__ out) {

@@ -23,6 +23,10 @@ int encode_tmap_bf16(CUtensorMap* map, const void* base, int rank, const uint64_
 int encode_tmap_f32(CUtensorMap* map, const void* base, int rank, const uint64_t* dims,
                     const uint64_t* strides_bytes /* rank-1 */, const uint32_t* box, int swizzle128);
 
+// aptai_gemm_wgrad_bf16 that writes only dw rows [0, out_rows): N (the dY columns the TMA reads) may be a padded width
+int wgrad_bf16_rows(const void* dy, int64_t dy_ld, const void* x, int64_t x_ld, int64_t M, int N, int K, float scale,
+                    float* dw, int64_t dw_ld, int out_rows, void* stream);
+
 #define APTAI_REQUIRE(cond, ...)              \
   do {                                        \
     if (!(cond)) {                            \

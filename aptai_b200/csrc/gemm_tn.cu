@@ -475,15 +475,10 @@ static int launch_tn(const CUtensorMap& ta, const CUtensorMap& tb, TnParams& p, 
   return after_launch("gemm_tn_wgrad");
 }
 
-}  // namespace aptai
-
-using namespace aptai;
-
-extern "C" int aptai_gemm_wgrad_bf16(const void* dy, int64_t dy_ld, const void* x, int64_t x_ld, int64_t M, int N,
-                                     int K, float scale, float* dw, int64_t dw_ld, void* stream) {
-  if (int rc = check_arch()) return rc;
+int wgrad_bf16_rows(const void* dy, int64_t dy_ld, const void* x, int64_t x_ld, int64_t M, int N, int K, float scale,
+                    float* dw, int64_t dw_ld, int out_rows, void* stream) {
   APTAI_REQUIRE(dy && x && dw, "gemm_wgrad: null pointer");
-  APTAI_REQUIRE(M >= 1 && N >= 1 && K >= 1, "gemm_wgrad: bad shape");
+  APTAI_REQUIRE(M >= 1 && N >= 1 && K >= 1 && out_rows >= 1 && out_rows <= N, "gemm_wgrad: bad shape");
   APTAI_REQUIRE(N % 8 == 0 && K % 8 == 0 && dy_ld % 8 == 0 && x_ld % 8 == 0 && dw_ld % 4 == 0,
                 "gemm_wgrad: N, K and the row pitches must be multiples of 8 (dw_ld of 4)");
   APTAI_REQUIRE(((reinterpret_cast<uintptr_t>(dy) | reinterpret_cast<uintptr_t>(x) | reinterpret_cast<uintptr_t>(dw)) & 15) == 0,
@@ -510,7 +505,7 @@ extern "C" int aptai_gemm_wgrad_bf16(const void* dy, int64_t dy_ld, const void* 
   p.b_col_kt = TN_BN; p.b_col_nt = 0; p.b_col_box = 64;
   p.b_row_kt = 0; p.b_row_box = 0;
   p.out_rows_per_tile = TN_BM;
-  p.out_rows = N; p.out_cols = K;
+  p.out_rows = out_rows; p.out_cols = K;
   p.ldo = dw_ld;
   p.out = dw;
   p.scale = scale;
@@ -522,6 +517,16 @@ extern "C" int aptai_gemm_wgrad_bf16(const void* dy, int64_t dy_ld, const void* 
     return launch_tn_pair(ta, tb, p, reinterpret_cast<cudaStream_t>(stream));
   }
   return launch_tn(ta, tb, p, reinterpret_cast<cudaStream_t>(stream));
+}
+
+}  // namespace aptai
+
+using namespace aptai;
+
+extern "C" int aptai_gemm_wgrad_bf16(const void* dy, int64_t dy_ld, const void* x, int64_t x_ld, int64_t M, int N,
+                                     int K, float scale, float* dw, int64_t dw_ld, void* stream) {
+  if (int rc = check_arch()) return rc;
+  return wgrad_bf16_rows(dy, dy_ld, x, x_ld, M, N, K, scale, dw, dw_ld, N, stream);
 }
 
 extern "C" int aptai_posconv_wgrad_bf16(const void* dy, const void* x_pad, int B, int T, int H, int groups, int taps,

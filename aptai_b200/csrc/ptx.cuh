@@ -550,4 +550,10 @@ __device__ __forceinline__ void pack32_h16(const float (&v)[32], uint4 (&o)[4], 
   }
 }
 
+// hi/lo bf16 pair of an fp32 value (accuracy-mode operands, csrc/accurate.cu): x = hi + lo to ~2^-17 relative
+__device__ __forceinline__ void split_bf16(float x, __nv_bfloat16& hi, __nv_bfloat16& lo) {
+  hi = __float2bfloat16_rn(x);
+  lo = __float2bfloat16_rn(x - __bfloat162float(hi));
+}
+
 }  // namespace aptai

@@ -78,8 +78,14 @@ class Force_APTAI(nn.Module):
         phn_pred_list = [np.asarray(s) for s in phn_seqs] if phn_seqs is not None else pr._decode(logits)
         phn_seq_lens = [len(l) for l in phn_pred_list]
         padded = []
+        n_emb = self.phn_emb_layer.num_embeddings
         for lst in phn_pred_list:
             assert len(lst) < self.max_phn_seq_len, "Need longer max phoneme sequence length."
+            # the cross-attention kernel indexes its embedding table with these ids unchecked
+            if len(lst) and (int(np.min(lst)) < 0 or int(np.max(lst)) >= n_emb):
+                raise ValueError(f"Force_APTAI: phoneme id {int(np.max(lst))} (or a negative one) outside the "
+                                 f"embedding table of {n_emb} entries (len(vocab)); the recogniser's vocabulary must "
+                                 "not be larger than Force_APTAI's")
             padded.append(np.pad(lst, (0, self.max_phn_seq_len - len(lst)), mode="constant"))
         phn_pred_seq = torch.tensor(np.stack(padded), dtype=torch.int32, device=dev)
         return h, logits, frame_seq_lens, phn_pred_list, phn_seq_lens, phn_pred_seq

@@ -64,6 +64,12 @@ PROTOTYPES = {
     "aptai_attention_fwd_v3": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_void_p]),
     "aptai_heads": (c_int, [c_void_p, c_i64, c_int, c_void_p, c_void_p, c_int, c_int, c_void_p, c_void_p, c_void_p,
                             c_int, c_int, c_void_p, c_void_p, c_void_p]),
+    "aptai_pr_head_wide_workspace_bytes": (c_size_t, [c_i64, c_int, c_int, c_int]),
+    "aptai_pr_head_wide": (c_int, [c_void_p, c_i64, c_int, c_void_p, c_void_p, c_int, c_void_p, c_i64, c_void_p,
+                                   c_size_t, c_void_p]),
+    "aptai_logits_rows": (c_int, [c_void_p, c_i64, c_int, c_i64, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p]),
+    "aptai_pr_head_wide_bwd": (c_int, [c_void_p, c_i64, c_int, c_void_p, c_int, c_void_p, c_i64, c_void_p, c_void_p,
+                                       c_void_p, c_void_p, c_size_t, c_void_p]),
     "aptai_lowpass_fir": (c_int, [c_void_p, c_int, c_int, c_int, c_void_p, c_int, c_void_p, c_void_p]),
     "aptai_softmax_rows": (c_int, [c_void_p, c_i64, c_int, c_int, c_void_p, c_void_p]),
     "aptai_tail": (c_int, [c_void_p, c_i64, c_int, c_void_p, c_void_p, c_float, c_void_p, c_void_p, c_int, c_int, c_void_p,

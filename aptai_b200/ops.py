@@ -418,6 +418,77 @@ def heads(h: torch.Tensor, wa, ba, act_a: int, wb, bb, act_b: int, want_argmax: 
     return oa, ob, am
 
 
+PR_HEAD_NARROW = 48        # head-B slots of aptai_heads: recogniser heads up to here run on that kernel
+PR_HEAD_MAX_VOCAB = 1024  # wide head (aptai_pr_head_wide, aptai_logits_rows): one row of logits per warp, 32 per lane
+
+
+def pr_head_wide(h: torch.Tensor, w: torch.Tensor, b: Optional[torch.Tensor], out: Optional[torch.Tensor] = None):
+    """Recogniser head h fp32 [rows,H] -> raw logits h @ w.T + b (fp32-accurate split-operand GEMM), 1 <= V <= 1024.
+    Returns the [rows, V] view of a pitched buffer (row stride >= 64*ceil(V/64)): `out` fp32 [rows, ld] if given,
+    else a new one; pass it to `logits_rows`."""
+    _req(h, F32, "h"); _req(w, F32, "w")
+    rows, H = h.shape
+    V = w.shape[0]
+    if w.shape[1] != H:
+        raise ValueError(f"pr_head_wide: weight {tuple(w.shape)} does not match h [{rows}, {H}]")
+    if b is not None:
+        _req(b, F32, "b")
+    if out is None:
+        out = torch.empty((rows, (V + 63) // 64 * 64), dtype=F32, device=h.device)
+    elif out.dtype != F32 or out.dim() != 2 or out.shape[0] != rows or out.stride(1) != 1:
+        raise ValueError("pr_head_wide: out must be fp32 [rows, ld] with unit column stride")
+    L = _lib.load()
+    nbytes = L.aptai_pr_head_wide_workspace_bytes(rows, H, V, 0)
+    if nbytes == 0:
+        raise ValueError(f"pr_head_wide: V={V}, H={H} unsupported (1 <= V <= {PR_HEAD_MAX_VOCAB}, H % 64 == 0)")
+    ws = torch.empty((nbytes,), dtype=torch.uint8, device=h.device)
+    check(L.aptai_pr_head_wide(h.data_ptr(), rows, H, w.data_ptr(), _ptr(b), V, out.data_ptr(), out.stride(0),
+                               ws.data_ptr(), nbytes, _stream()), "pr_head_wide")
+    return out[:, :V]
+
+
+def logits_rows(x: torch.Tensor, *, want_logits: bool = True, want_argmax: bool = False, want_logp: bool = False,
+                want_prob: bool = False):
+    """One pass over fp32 rows x [rows, V] (V <= 1024; any row stride, unit column stride) -> (logits contiguous
+    [rows, V] | None, first-max argmax int64 [rows] | None, log_softmax | None, softmax | None)."""
+    if not x.is_cuda or x.dtype != F32 or x.dim() != 2 or x.stride(1) != 1:
+        raise ValueError("logits_rows: x must be a CUDA fp32 [rows, V] tensor with unit column stride")
+    rows, V = x.shape
+    dev = x.device
+    new = lambda on, dt=F32, shape=(rows, V): torch.empty(shape, dtype=dt, device=dev) if on else None
+    lg, am, lp, pr = new(want_logits), new(want_argmax, I64, (rows,)), new(want_logp), new(want_prob)
+    check(_lib.load().aptai_logits_rows(x.data_ptr(), rows, V, x.stride(0), _ptr(lg), _ptr(am), _ptr(lp), _ptr(pr),
+                                        _stream()), "logits_rows")
+    return lg, am, lp, pr
+
+
+def pr_head_wide_bwd(h: torch.Tensor, w: torch.Tensor, d_logits: torch.Tensor, dw: Optional[torch.Tensor],
+                     db: Optional[torch.Tensor], want_dh: bool = True) -> Optional[torch.Tensor]:
+    """Backward of `pr_head_wide`: returns dh = d_logits @ w (fp32 [rows,H]) and accumulates dw += d_logits.T @ h,
+    db += d_logits.sum(0) (either may be None).  d_logits fp32 [rows, V], any row stride, unit column stride."""
+    _req(h, F32, "h"); _req(w, F32, "w")
+    rows, H = h.shape
+    V = w.shape[0]
+    if (d_logits.dtype != F32 or not d_logits.is_cuda or tuple(d_logits.shape) != (rows, V)
+            or d_logits.stride(1) != 1):
+        raise ValueError(f"pr_head_wide_bwd: d_logits must be CUDA fp32 [{rows}, {V}] with unit column stride")
+    if dw is not None:
+        _req(dw, F32, "dw")
+        assert tuple(dw.shape) == (V, H)
+    if db is not None:
+        _req(db, F32, "db")
+        assert db.numel() == V
+    dh = torch.empty_like(h) if want_dh else None
+    L = _lib.load()
+    nbytes = L.aptai_pr_head_wide_workspace_bytes(rows, H, V, 1)
+    if nbytes == 0:
+        raise ValueError(f"pr_head_wide_bwd: V={V}, H={H} unsupported (1 <= V <= {PR_HEAD_MAX_VOCAB}, H % 64 == 0)")
+    ws = torch.empty((nbytes,), dtype=torch.uint8, device=h.device)
+    check(L.aptai_pr_head_wide_bwd(h.data_ptr(), rows, H, w.data_ptr(), V, d_logits.data_ptr(), d_logits.stride(0),
+                                   _ptr(dh), _ptr(dw), _ptr(db), ws.data_ptr(), nbytes, _stream()), "pr_head_wide_bwd")
+    return dh
+
+
 def tail(h: torch.Tensor, ln_gamma, ln_beta, eps: float, wa, ba, act_a: int, wb, bb, act_b: int, *,
          want_argmax: bool = True, want_logp: bool = False, want_h_norm: bool = False):
     """Fused tail: (final LayerNorm) -> heads A / B -> argmax -> log_softmax.  h fp32 [rows,H].

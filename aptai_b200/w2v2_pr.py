@@ -60,6 +60,21 @@ class _HiddenStatesFn(torch.autograd.Function):
         return (None,) * (4 + len(idx))
 
 
+def _head_fwd(hm, w, b):
+    """pr_head logits fp32 [rows, V] of h fp32 [rows, H]: the fused heads kernel up to ops.PR_HEAD_NARROW classes, the
+    fp32-accurate tensor-core head beyond (ops.pr_head_wide + one pass of ops.logits_rows)."""
+    if w.shape[0] <= ops.PR_HEAD_NARROW:
+        return ops.heads(hm, None, None, 0, w, b, ops.ACT_NONE, want_argmax=False)[1]
+    return ops.logits_rows(ops.pr_head_wide(hm, w, b))[0]
+
+
+def _head_bwd(hm, w, d_lg, dw, db):
+    """dh of `_head_fwd` (fp32 [rows, H]); dw / db accumulate."""
+    if w.shape[0] <= ops.PR_HEAD_NARROW:
+        return ops.heads_bwd(hm, None, None, 0, None, None, d_lg, w, ops.ACT_NONE, dw, db)
+    return ops.pr_head_wide_bwd(hm, w, d_lg, dw, db)
+
+
 class _HeadFn(torch.autograd.Function):
     """pr_head (Linear H -> vocab) through the heads kernels, differentiable w.r.t. its input and parameters."""
 
@@ -68,8 +83,7 @@ class _HeadFn(torch.autograd.Function):
         B, T, H = h.shape
         hm = h.detach().reshape(B * T, H).float().contiguous()
         w = weight.detach().float().contiguous()
-        _, logits, _ = ops.heads(hm, None, None, 0, w, bias.detach().float().contiguous(), ops.ACT_NONE,
-                                 want_argmax=False)
+        logits = _head_fwd(hm, w, bias.detach().float().contiguous())
         ctx.save_for_backward(hm, w)
         return logits.view(B, T, -1)
 
@@ -79,8 +93,7 @@ class _HeadFn(torch.autograd.Function):
         B, T, V = d_logits.shape
         dw = torch.zeros_like(w)
         db = torch.zeros((V,), dtype=torch.float32, device=w.device)
-        dh = ops.heads_bwd(hm, None, None, 0, None, None, d_logits.reshape(B * T, V).float().contiguous(), w,
-                           ops.ACT_NONE, dw, db)
+        dh = _head_bwd(hm, w, d_logits.reshape(B * T, V).float().contiguous(), dw, db)
         return dh.view(B, T, -1), dw, db
 
 
@@ -94,6 +107,10 @@ class Wav2Vec2_PR(nn.Module):
     def __init__(self, pretrain_cfg, cache_dir, huggingface_model_id, vocab=None,
                  phoneme_decoder: Optional[Callable] = None):
         super().__init__()
+        vocab_size = int(getattr(pretrain_cfg, "vocab_size", 0))
+        if vocab_size > ops.PR_HEAD_MAX_VOCAB:
+            raise ValueError(f"Wav2Vec2_PR: vocab_size={vocab_size} exceeds the recogniser head's limit of "
+                             f"{ops.PR_HEAD_MAX_VOCAB} symbols")
         self.cache_dir = cache_dir
         self.huggingface_model_id = huggingface_model_id
         self.pretrain_cfg = pretrain_cfg
@@ -121,8 +138,7 @@ class Wav2Vec2_PR(nn.Module):
     def _head(self, h):
         B, T, H = h.shape
         f = lambda p: p.detach().float().contiguous()
-        _, logits, _ = ops.heads(h.reshape(B * T, H).contiguous(), None, None, 0, f(self.pr_head.weight),
-                                 f(self.pr_head.bias), ops.ACT_NONE, want_argmax=False)
+        logits = _head_fwd(h.reshape(B * T, H).contiguous(), f(self.pr_head.weight), f(self.pr_head.bias))
         return logits.view(B, T, -1)
 
     def enable_data_parallel(self, group=None, layers_per_bucket: int = 4, broadcast: bool = True,
@@ -200,8 +216,7 @@ class Wav2Vec2_PR(nn.Module):
 
             def run_backward(grad_out):
                 d_lg = (r["grad"] * grad_out.detach().to(device=dev, dtype=torch.float32)).view(B * T, V).contiguous()
-                dh = ops.heads_bwd(hm, None, None, 0, None, None, d_lg, w, ops.ACT_NONE, gb.view("pr_head.weight"),
-                                   gb.view("pr_head.bias"))
+                dh = _head_bwd(hm, w, d_lg, gb.view("pr_head.weight"), gb.view("pr_head.bias"))
                 if p_fin > 0:
                     ops.dropout(dh, p_fin, s_fin, out_f32=dh)
                 red = getattr(self, "_reducer", None)

@@ -177,6 +177,27 @@ int aptai_heads(const float* h, int64_t rows, int H, const float* wa, const floa
                 float* out_a, const float* wb, const float* bb, int nb, int act_b, float* out_b,
                 int64_t* argmax_b, void* stream);
 
+/* Phoneme-recogniser head wider than aptai_heads' 48 head-B slots (models/w2v2_pr.py:47 pr_head = Linear(H, V)),
+ * 1 <= V <= 1024, H a multiple of 64 (csrc/pr_head.cu).  fp32 accuracy on the tensor cores: the split-operand GEMM of
+ * the accuracy mode, [h_hi | h_lo | h_hi] . [W_hi | W_hi | W_lo]^T + b (relative error ~2^-17 of |h| |W|).
+ * Padding and pitch: W gets zero rows up to Vp = 64 * ceil(V / 64) (a GEMM tile width), and `out` is fp32 [rows][ld_out]
+ * with ld_out >= Vp, ld_out % 8 == 0: columns [0, V) hold the logits, [V, Vp) are written with zeros, columns >= Vp
+ * are not touched.  b may be NULL.  ws: aptai_pr_head_wide_workspace_bytes(rows, H, V, 0) bytes, 256-byte aligned.
+ * Nothing here allocates or synchronises (CUDA-graph capturable): the weight split runs on every call. */
+size_t aptai_pr_head_wide_workspace_bytes(int64_t rows, int H, int V, int backward);
+int aptai_pr_head_wide(const float* h, int64_t rows, int H, const float* w, const float* b, int V, float* out,
+                       int64_t ld_out, void* ws, size_t ws_bytes, void* stream);
+/* One pass over fp32 rows x [rows][ldx] (columns [0, V), V <= 1024, one warp per row): any of the compact logits
+ * fp32 [rows][V], the first-max argmax int64 [rows], log_softmax and softmax fp32 [rows][V] (each may be NULL). */
+int aptai_logits_rows(const float* x, int64_t rows, int V, int64_t ldx, float* logits, int64_t* argmax, float* logp,
+                      float* prob, void* stream);
+/* Backward of aptai_pr_head_wide: d_logits fp32 [rows][V] with row pitch ld_d >= V;
+ * dh = d_logits W (written, fp32 [rows][H]), dw += d_logits^T h (fp32 [V][H]), db += column sums (fp32 [V]); each
+ * output may be NULL.  Split-operand GEMMs (K = 3 Vp for dh; three MN-major wgrad products for dw).
+ * ws: aptai_pr_head_wide_workspace_bytes(rows, H, V, 1) bytes, 256-byte aligned. */
+int aptai_pr_head_wide_bwd(const float* h, int64_t rows, int H, const float* w, int V, const float* d_logits,
+                           int64_t ld_d, float* dh, float* dw, float* db, void* ws, size_t ws_bytes, void* stream);
+
 /* LowPassFilterLayer (models/modules.py:46-61): per channel 51-tap FIR, zero 'same' padding along T, fp64
  * accumulation of the fp64 taps, fp32 in/out [B][T][C]. */
 int aptai_lowpass_fir(const float* x, int B, int T, int C, const double* taps, int ntaps, float* y, void* stream);
