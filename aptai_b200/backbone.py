@@ -593,7 +593,7 @@ class Wav2Vec2Backbone(nn.Module):
         # Without hidden dropout the gradient of out-proj's / FFN2's OUTPUT is the residual-stream gradient a LayerNorm
         # backward has just produced: that kernel accumulates its column sums (the bias gradient) on the way out
         # (`dcolsum`), which saves the colsum launch that would re-read the tensor.
-        fuse_bias = p_h == 0 and bool(ops.FUSED_BIAS_COLSUM)
+        fuse_bias = p_h == 0
 
         def masked16(d32, d16, li, site):
             """bf16 gradient w.r.t. the input of a hidden-dropout site (same mask as the forward)."""
@@ -814,30 +814,16 @@ class Wav2Vec2Backbone(nn.Module):
             # every activation of a 75 k-row batch (h 300 MB, qkv 450 MB, u 600 MB) exceeds the 126 MB L2: consecutive
             # kernels walk their rows in ALTERNATING directions, so each one starts on the rows its producer wrote last
             serp = ops.Serpentine()
-            # the LayerNorm behind each in-place residual update (out-proj -> LN2, FFN2 -> the next layer's LN1) runs
-            # inside that GEMM launch, on rows still in L2 (ops.linear row_ln); only layer 0's LN1 is a launch of its own
-            fuse = ops.FUSED_ROW_LN and H in (768, 1024) and not collect_hidden
-            x = None
-            for i, lw in enumerate(P.layers):
+            for lw in P.layers:
                 if collect_hidden:
                     hidden.append(h.view(B, T, H).clone())
-                if x is None:
-                    serp(); _, x = ops.layernorm(h, lw.ln1_w, lw.ln1_b, eps, out16_dtype=X16)
+                serp(); _, x = ops.layernorm(h, lw.ln1_w, lw.ln1_b, eps, out16_dtype=X16)
                 serp(); _, qkv = ops.linear(x, lw.qkv_w, lw.qkv_b)
                 serp(); ctx = ops.attention(qkv, frame_lens, B, T, heads)
-                if fuse:
-                    nxt = P.layers[i + 1] if i + 1 < len(P.layers) else None
-                    serp(); _, x = ops.linear(ctx, lw.o_w, lw.o_b, residual=h, out_f32=h, want_bf16=False,
-                                              row_ln=(lw.ln2_w, lw.ln2_b, eps))
-                    serp(); _, u = ops.linear(x, lw.ff1_w, lw.ff1_b, act=1)
-                    serp(); _, x = ops.linear(u, lw.ff2_w, lw.ff2_b, residual=h, out_f32=h, want_bf16=False,
-                                              row_ln=(nxt.ln1_w, nxt.ln1_b, eps) if nxt is not None else None)
-                else:
-                    serp(); ops.linear(ctx, lw.o_w, lw.o_b, residual=h, out_f32=h, want_bf16=False)
-                    serp(); _, x = ops.layernorm(h, lw.ln2_w, lw.ln2_b, eps, out16_dtype=X16)
-                    serp(); _, u = ops.linear(x, lw.ff1_w, lw.ff1_b, act=1)
-                    serp(); ops.linear(u, lw.ff2_w, lw.ff2_b, residual=h, out_f32=h, want_bf16=False)
-                    x = None
+                serp(); ops.linear(ctx, lw.o_w, lw.o_b, residual=h, out_f32=h, want_bf16=False)
+                serp(); _, x = ops.layernorm(h, lw.ln2_w, lw.ln2_b, eps, out16_dtype=X16)
+                serp(); _, u = ops.linear(x, lw.ff1_w, lw.ff1_b, act=1)
+                serp(); ops.linear(u, lw.ff2_w, lw.ff2_b, residual=h, out_f32=h, want_bf16=False)
             serp.done()
             if final_ln or collect_hidden:
                 last, _ = ops.layernorm(h, P.enc_ln_w, P.enc_ln_b, eps, want_f32=True, want_bf16=False)

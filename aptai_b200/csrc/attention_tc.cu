@@ -16,8 +16,6 @@
 #include "common.h"
 #include "ptx.cuh"
 
-#include <stdlib.h>
-
 namespace aptai {
 
 constexpr int AQ = 128;                 // query rows per work item
@@ -397,15 +395,7 @@ static int attention_fwd_impl(const void* qkv, void* ctx, float* lse, const int3
     }
     attr_set = true;
   }
-  static int ctas_per_sm = 0;
-  if (ctas_per_sm == 0) {
-    int n = 0;
-    cudaError_t e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&n, kern, ATC_THREADS, ATC_SMEM);
-    if (getenv("APTAI_DEBUG"))
-      fprintf(stderr, "aptai attention: occupancy query -> %d CTAs per SM (%s)\n", n, cudaGetErrorString(e));
-    cudaGetLastError();
-    ctas_per_sm = 2;      // two CTAs per SM are intended (80 KB smem, 256 TMEM columns, <= 128 registers each)
-  }
+  const int ctas_per_sm = 2;      // two CTAs per SM are intended (80 KB smem, 256 TMEM columns, <= 128 registers each)
   const int grid = p.items < ctas_per_sm * num_sms() ? p.items : ctas_per_sm * num_sms();
   kern<<<grid, ATC_THREADS, ATC_SMEM, reinterpret_cast<cudaStream_t>(stream)>>>(tmq, tmkv, p);
   return after_launch("attention_tc");

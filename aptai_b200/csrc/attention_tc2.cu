@@ -17,10 +17,10 @@
 // instead of being held in 64 registers, which keeps the kernel at two CTAs per SM.
 // Same contract as aptai_attention_fwd: q pre-scaled by head_dim^-0.5, every query row computed, keys >= key_len[b]
 // masked, lazy rescaling of O (threshold 2^8), optional log2-domain lse output for the backward pass.
+// It serves the training forward with dropout on the attention probabilities (aptai_attention_fwd_dropout; at p = 0
+// the mask keeps every element and the scale is 1).
 #include "common.h"
 #include "ptx.cuh"
-
-#include <stdlib.h>
 
 namespace aptai {
 
@@ -87,7 +87,7 @@ __device__ __forceinline__ void a2_tmem_st32(uint32_t taddr, const uint32_t (&r)
 // exp pass over one FULL 64-key tile of one query row: p = exp2(s*log2e - m_used) -> bf16 -> shared memory (K-major
 // SWIZZLE_128B), row sum, optionally the raw row maximum.  TMEM is read in four 16-column chunks, the load of chunk
 // c+1 in flight while chunk c is processed; packed fp32x2 math (FFMA2 / FADD2) for the exponent argument and the sum.
-template <bool TRACK_MAX, bool DROP>
+template <bool TRACK_MAX>
 __device__ __forceinline__ void a2_exp_tile_full(uint32_t ts, float m_used, uint8_t* prow, int row, float& rowsum,
                                                  float& rawmax, const A2Drop& dc, int key0) {
   const uint64_t l2e = f32x2_pack(A2_LOG2E, A2_LOG2E), nm = f32x2_pack(-m_used, -m_used);
@@ -110,14 +110,10 @@ __device__ __forceinline__ void a2_exp_tile_full(uint32_t ts, float m_used, uint
         const float p0 = a2_ex2(a0), p1 = a2_ex2(a1);
         if (i & 1) acc1 = f32x2_add(acc1, f32x2_pack(p0, p1));
         else acc0 = f32x2_add(acc0, f32x2_pack(p0, p1));
-        if (DROP) {
-          const uint32_t kk = key0 + chunk * 16 + u * 8 + 2 * i;
-          const float d0 = attn_drop_keep(dc.seed_bh, dc.q, kk, dc.T, dc.thresh24) ? p0 * dc.inv_keep : 0.f;
-          const float d1 = attn_drop_keep(dc.seed_bh, dc.q, kk + 1, dc.T, dc.thresh24) ? p1 * dc.inv_keep : 0.f;
-          wv[i] = pack_bf16(d0, d1);
-        } else {
-          wv[i] = pack_bf16(p0, p1);
-        }
+        const uint32_t kk = key0 + chunk * 16 + u * 8 + 2 * i;
+        const float d0 = attn_drop_keep(dc.seed_bh, dc.q, kk, dc.T, dc.thresh24) ? p0 * dc.inv_keep : 0.f;
+        const float d1 = attn_drop_keep(dc.seed_bh, dc.q, kk + 1, dc.T, dc.thresh24) ? p1 * dc.inv_keep : 0.f;
+        wv[i] = pack_bf16(d0, d1);
       }
       *reinterpret_cast<uint4*>(prow + (((chunk * 2 + u) ^ (row & 7)) << 4)) = make_uint4(wv[0], wv[1], wv[2], wv[3]);
     }
@@ -140,7 +136,6 @@ __device__ __forceinline__ void a2_exp_tile_full(uint32_t ts, float m_used, uint
   rawmax = fmaxf(m0, m1);
 }
 
-template <bool DROP>
 __global__ void __launch_bounds__(A2_THREADS, 2)
 attention_tc2_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constant__ CUtensorMap tmKV,
                      const Attn2Params p) {
@@ -323,7 +318,7 @@ attention_tc2_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_const
       const int n = (klen + A2_K - 1) / A2_K;
       float m_used = -INFINITY, l = 0.f;
       A2Drop dc;
-      dc.seed_bh = DROP ? attn_drop_seed_bh(p.drop_seed, static_cast<uint32_t>(bh)) : 0u;
+      dc.seed_bh = attn_drop_seed_bh(p.drop_seed, static_cast<uint32_t>(bh));
       dc.q = static_cast<uint32_t>(qp * 2 * A2_Q + t * A2_Q + row);
       dc.T = static_cast<uint32_t>(p.T);
       dc.thresh24 = p.drop_thresh24;
@@ -347,7 +342,7 @@ attention_tc2_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_const
         if (valid >= A2_K && j > 0) {
           mbar_wait(&p_empty[t], (g - 1) & 1);           // P_t free: P_t(j-1) V_(j-1) has completed
           float rsum, rmax;
-          a2_exp_tile_full<true, DROP>(ts, m_used, prow, row, rsum, rmax, dc, j * A2_K);
+          a2_exp_tile_full<true>(ts, m_used, prow, row, rsum, rmax, dc, j * A2_K);
           if (!__any_sync(0xffffffffu, rmax * A2_LOG2E > m_used + A2_RESCALE)) {
             l += rsum;
             done = true;
@@ -410,7 +405,7 @@ attention_tc2_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_const
         float rs0 = 0.f, rs1 = 0.f, rs2 = 0.f, rs3 = 0.f;
         if (valid >= A2_K) {
           float rmax_unused;
-          a2_exp_tile_full<false, DROP>(ts, m_used, prow, row, rs0, rmax_unused, dc, j * A2_K);
+          a2_exp_tile_full<false>(ts, m_used, prow, row, rs0, rmax_unused, dc, j * A2_K);
         } else {
           const int ncol16 = (valid + 15) >> 4;
 #pragma unroll
@@ -428,12 +423,10 @@ attention_tc2_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_const
                   if (c * 32 + u8 * 8 + i >= valid) pv[i] = 0.f;
                 }
                 rs0 += pv[0] + pv[4]; rs1 += pv[1] + pv[5]; rs2 += pv[2] + pv[6]; rs3 += pv[3] + pv[7];
-                if (DROP) {
 #pragma unroll
-                  for (int i = 0; i < 8; ++i)
-                    pv[i] = attn_drop_keep(dc.seed_bh, dc.q, j * A2_K + c * 32 + u8 * 8 + i, dc.T, dc.thresh24)
-                                ? pv[i] * dc.inv_keep : 0.f;
-                }
+                for (int i = 0; i < 8; ++i)
+                  pv[i] = attn_drop_keep(dc.seed_bh, dc.q, j * A2_K + c * 32 + u8 * 8 + i, dc.T, dc.thresh24)
+                              ? pv[i] * dc.inv_keep : 0.f;
                 const int unit = c * 4 + u8;
                 if ((unit >> 1) < ncol16)
                   *reinterpret_cast<uint4*>(prow + ((unit ^ (row & 7)) << 4)) =
@@ -491,8 +484,8 @@ attention_tc2_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_const
 
 using namespace aptai;
 
-static int attention_v2_impl(const void* qkv, void* ctx, float* lse, const int32_t* key_len, int B, int T, int heads,
-                             float drop_p, uint64_t drop_seed, void* stream) {
+extern "C" int aptai_attention_fwd_dropout(const void* qkv, void* ctx, float* lse, const int32_t* key_len, int B, int T,
+                                           int heads, float drop_p, uint64_t drop_seed, void* stream) {
   if (int rc = check_arch()) return rc;
   APTAI_REQUIRE(qkv && ctx && key_len, "attention_v2: null pointer");
   APTAI_REQUIRE(B >= 1 && T >= 1 && heads >= 1, "attention_v2: bad shape");
@@ -522,34 +515,19 @@ static int attention_v2_impl(const void* qkv, void* ctx, float* lse, const int32
   p.drop_seed = drop_seed;
   static bool attr_set = false;
   if (!attr_set) {
-    for (int v = 0; v < 2; ++v) {
-      const void* fn = v ? reinterpret_cast<const void*>(attention_tc2_kernel<true>)
-                         : reinterpret_cast<const void*>(attention_tc2_kernel<false>);
-      cudaFuncSetAttribute(fn, cudaFuncAttributePreferredSharedMemoryCarveout, 100);
-      cudaError_t e = cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, A2_SMEM);
-      if (e != cudaSuccess) {
-        set_error("attention_v2: cudaFuncSetAttribute: %s", cudaGetErrorString(e));
-        return static_cast<int>(e);
-      }
+    cudaFuncSetAttribute(attention_tc2_kernel, cudaFuncAttributePreferredSharedMemoryCarveout, 100);
+    cudaError_t e = cudaFuncSetAttribute(attention_tc2_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, A2_SMEM);
+    if (e != cudaSuccess) {
+      set_error("attention_v2: cudaFuncSetAttribute: %s", cudaGetErrorString(e));
+      return static_cast<int>(e);
     }
     attr_set = true;
   }
   const int slots = 2 * num_sms();
   const int grid = p.items < slots ? p.items : slots;
   cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
-  if (drop_p > 0.f) attention_tc2_kernel<true><<<grid, A2_THREADS, A2_SMEM, st>>>(tmq, tmkv, p);
-  else attention_tc2_kernel<false><<<grid, A2_THREADS, A2_SMEM, st>>>(tmq, tmkv, p);
+  attention_tc2_kernel<<<grid, A2_THREADS, A2_SMEM, st>>>(tmq, tmkv, p);
   return after_launch("attention_tc2");
-}
-
-extern "C" int aptai_attention_fwd_v2(const void* qkv, void* ctx, float* lse, const int32_t* key_len, int B, int T,
-                                      int heads, void* stream) {
-  return attention_v2_impl(qkv, ctx, lse, key_len, B, T, heads, 0.f, 0, stream);
-}
-
-extern "C" int aptai_attention_fwd_dropout(const void* qkv, void* ctx, float* lse, const int32_t* key_len, int B, int T,
-                                           int heads, float drop_p, uint64_t drop_seed, void* stream) {
-  return attention_v2_impl(qkv, ctx, lse, key_len, B, T, heads, drop_p, drop_seed, stream);
 }
 
 namespace aptai {

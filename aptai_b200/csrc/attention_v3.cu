@@ -22,7 +22,7 @@
 //     box 64 x 32 rows: clipped at the utterance's last frame, no per-row predicate, no barrier between warps); the
 //     read-out of an item's O is deferred into the first key tile of the next item, where the wait for the item's
 //     last P V hides behind that tile's softmax.
-// Same contract as aptai_attention_fwd_v2: q pre-scaled by head_dim^-0.5, keys >= key_len[b] masked, lazy rescaling
+// Same contract as aptai_attention_fwd: q pre-scaled by head_dim^-0.5, keys >= key_len[b] masked, lazy rescaling
 // of O (threshold 2^8), optional log2-domain lse output for the backward pass.
 #include "common.h"
 #include "ptx.cuh"
@@ -45,12 +45,12 @@ constexpr uint32_t A3_TO = 2 * A3_NBUF * A3_K;   // O_t at 384 + t*64
 constexpr uint32_t A3_TCOLS = 512;
 constexpr float A3_LOG2E = 1.4426950408889634f;
 constexpr float A3_RESCALE = 8.0f;
+constexpr int A3_POLY8 = 3;                // of every 8 exponential pairs, this many are evaluated on the FMA pipe
 
 struct Attn3Params {
   const int* key_len;
   float* lse;
   int B, T, heads, n_qp, items, per_cta;
-  int idle_ns;              // issuer back-off when nothing is ready (0: poll hot)
   int reverse;              // aptai_set_traversal: utterances from the last to the first
 };
 
@@ -188,10 +188,9 @@ __device__ __forceinline__ void a3_ex2_poly2(float x0, float x1, float& p0, floa
   p1 = __uint_as_float(__float_as_uint(q1) + (__float_as_uint(r1) << 23));
 }
 
-// POLY8 of every 8 exponential PAIRS go to the FMA pipe, the rest to the MUFU; FP16: q / k / v, P and the context
-// are IEEE fp16 instead of bf16 (same tensor-core rate, three more mantissa bits; P <= 1 and the 2^8 lazy-rescale
-// window keep the unnormalised P far inside fp16's range)
-template <int POLY8, bool FP16>
+// FP16: q / k / v, P and the context are IEEE fp16 instead of bf16 (same tensor-core rate, three more mantissa bits;
+// P <= 1 and the 2^8 lazy-rescale window keep the unnormalised P far inside fp16's range)
+template <bool FP16>
 __global__ void __launch_bounds__(A3_THREADS, 1)
 attention_v3_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constant__ CUtensorMap tmKV,
                     const __grid_constant__ CUtensorMap tmO, const Attn3Params p) {
@@ -366,14 +365,8 @@ attention_v3_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_consta
             }
           }
         }
-        if (progress) {
-          idle = 0;
-        } else {
-          // nothing ready: sleep instead of polling hot — the issuer shares its scheduler with two softmax warps, and
-          // every group advances at the pace of its slowest warp (three S buffers of look-ahead absorb the delay)
-          if (p.idle_ns > 0) __nanosleep(p.idle_ns);
-          ++idle;
-        }
+        if (progress) idle = 0;
+        else ++idle;
         if (idle > (APTAI_SPIN_LIMIT >> 4)) {
           if (lane == 0) printf("aptai attention v3: MMA issuer %d timed out (block %d)\n", t, (int)blockIdx.x);
           __trap();
@@ -516,7 +509,7 @@ attention_v3_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_consta
         for (int i = 0; i < 32; ++i) {
           float a0, a1, p0, p1;
           f32x2_unpack(f32x2_fma(f32x2_pack(__uint_as_float(s[2 * i]), __uint_as_float(s[2 * i + 1])), l2e, nm), a0, a1);
-          if ((i & 7) < POLY8) {
+          if ((i & 7) < A3_POLY8) {
             a3_ex2_poly2(a0, a1, p0, p1);
           } else {
             p0 = a3_ex2(a0);
@@ -554,10 +547,10 @@ attention_v3_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_consta
 
 using namespace aptai;
 
-template <int POLY8, bool FP16>
+template <bool FP16>
 static int launch_attention_v3(const CUtensorMap& tq, const CUtensorMap& tkv, const CUtensorMap& to,
                                const Attn3Params& p, cudaStream_t st) {
-  auto kern = attention_v3_kernel<POLY8, FP16>;
+  auto kern = attention_v3_kernel<FP16>;
   static bool attr_set = false;
   if (!attr_set) {
     cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, A3_SMEM);
@@ -573,7 +566,7 @@ static int launch_attention_v3(const CUtensorMap& tq, const CUtensorMap& tkv, co
 }
 
 extern "C" int aptai_attention_fwd_v3(const void* qkv, void* ctx, float* lse, const int32_t* key_len, int B, int T,
-                                      int heads, int poly8, void* stream) {
+                                      int heads, int half_fmt, void* stream) {
   if (int rc = check_arch()) return rc;
   APTAI_REQUIRE(qkv && ctx && key_len, "attention_v3: null pointer");
   APTAI_REQUIRE(B >= 1 && T >= 1 && heads >= 1, "attention_v3: bad shape");
@@ -601,13 +594,6 @@ extern "C" int aptai_attention_fwd_v3(const void* qkv, void* ctx, float* lse, co
   p.items = B * heads * p.n_qp;
   p.per_cta = (p.items + num_sms() - 1) / num_sms();
   cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
-  p.idle_ns = (poly8 >> 8) & 0xffff;
   p.reverse = traversal_reverse();
-  if (poly8 & (1 << 24)) return launch_attention_v3<3, true>(tmq, tmkv, tmo, p, st);     // fp16 operands
-  switch (poly8 & 0xff) {
-    case 0: return launch_attention_v3<0, false>(tmq, tmkv, tmo, p, st);
-    case 2: return launch_attention_v3<2, false>(tmq, tmkv, tmo, p, st);
-    case 4: return launch_attention_v3<4, false>(tmq, tmkv, tmo, p, st);
-    default: return launch_attention_v3<3, false>(tmq, tmkv, tmo, p, st);
-  }
+  return half_fmt ? launch_attention_v3<true>(tmq, tmkv, tmo, p, st) : launch_attention_v3<false>(tmq, tmkv, tmo, p, st);
 }

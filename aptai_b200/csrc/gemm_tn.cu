@@ -17,8 +17,6 @@
 #include "common.h"
 #include "ptx.cuh"
 
-#include <stdlib.h>
-
 namespace aptai {
 
 constexpr int TN_BM = 128;       // dY columns per tile  (UMMA M)
@@ -510,8 +508,7 @@ int wgrad_bf16_rows(const void* dy, int64_t dy_ld, const void* x, int64_t x_ld, 
   p.out = dw;
   p.scale = scale;
   p.conv_P = 0; p.conv_cblks = 0;
-  static const bool force_single = getenv("APTAI_WGRAD_SINGLE") != nullptr;      // A/B switch for profiles/
-  if (!force_single && N >= 256 && K >= 256) {
+  if (N >= 256 && K >= 256) {
     p.n_tiles = (N + 255) / 256;
     p.k_tiles = (K + 255) / 256;
     return launch_tn_pair(ta, tb, p, reinterpret_cast<cudaStream_t>(stream));

@@ -29,8 +29,6 @@ class GemmArgs(C.Structure):
         ("out_f32", c_void_p), ("out_bf16", c_void_p), ("ldo", c_i64), ("out_seg_stride", c_i64),
         ("seg_valid_rows", c_void_p), ("mask_seg_rows", C.c_int32), ("act", C.c_int32), ("ln", C.c_int32), ("ln_eps", c_float), ("cta_pair", C.c_int32), ("half_fmt", C.c_int32),
         ("aux", c_void_p), ("out_pre", c_void_p),
-        ("row_ln_out", c_void_p), ("row_ln_gamma", c_void_p), ("row_ln_beta", c_void_p), ("row_ln_counters", c_void_p),
-        ("row_ln_eps", c_float),
     ]
 
 
@@ -60,7 +58,6 @@ PROTOTYPES = {
                                        c_void_p]),
     "aptai_attention_fwd_fmt": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_void_p]),
     "aptai_attention_fwd": (c_int, [c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_void_p]),
-    "aptai_attention_fwd_v2": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_void_p]),
     "aptai_attention_fwd_v3": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_void_p]),
     "aptai_heads": (c_int, [c_void_p, c_i64, c_int, c_void_p, c_void_p, c_int, c_int, c_void_p, c_void_p, c_void_p,
                             c_int, c_int, c_void_p, c_void_p, c_void_p]),

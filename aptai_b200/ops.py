@@ -74,12 +74,10 @@ def linear(a: torch.Tensor, w: torch.Tensor, bias: Optional[torch.Tensor] = None
            out_bf16: Optional[torch.Tensor] = None, want_f32: bool = False, want_bf16: bool = True,
            seg_rows: Optional[int] = None, seg_valid_rows: Optional[torch.Tensor] = None,
            block_n: int = 0, cta_pair: int = 0, aux: Optional[torch.Tensor] = None,
-           out_pre: Optional[torch.Tensor] = None, row_ln=None):
+           out_pre: Optional[torch.Tensor] = None):
     """out = epilogue(a @ w.T): a bf16 [M,K], w bf16 [N,K] (nn.Linear layout), bias fp32 [N].
 
     seg_rows / seg_valid_rows: rows are grouped in segments of seg_rows; rows >= seg_valid_rows[s] are written as 0.
-    row_ln = (gamma, beta, eps[, out16]): with the in-place residual update (residual is out_f32, no 16-bit output)
-    the same launch also writes LayerNorm(updated rows) in a's dtype — returned in place of the 16-bit output.
     """
     fmt = _h16(a, "a")
     if _h16(w, "w") != fmt:
@@ -116,36 +114,8 @@ def linear(a: torch.Tensor, w: torch.Tensor, bias: Optional[torch.Tensor] = None
         if out_pre.shape != (M, N) or out_pre.dtype != a.dtype:
             raise ValueError("linear: out_pre must match the 16-bit output")
         g.out_pre = out_pre.data_ptr()
-    if row_ln is not None:
-        if out_bf16 is not None or residual is None or out_f32 is None or residual.data_ptr() != out_f32.data_ptr():
-            raise ValueError("linear: row_ln rides on the in-place residual update (residual is out_f32, want_bf16=False)")
-        gamma, beta, eps = row_ln[0], row_ln[1], float(row_ln[2])
-        ln_out = row_ln[3] if len(row_ln) > 3 and row_ln[3] is not None else torch.empty((M, N), dtype=a.dtype,
-                                                                                         device=a.device)
-        if ln_out.shape != (M, N) or ln_out.dtype != a.dtype or not ln_out.is_contiguous():
-            raise ValueError("linear: row_ln output must be a contiguous [M, N] tensor of a's dtype")
-        cnt = _row_ln_counters(a.device, 2 * ((M + 255) // 256))
-        g.row_ln_out = ln_out.data_ptr()
-        g.row_ln_gamma = _req(gamma, F32, "row_ln gamma").data_ptr()
-        g.row_ln_beta = _req(beta, F32, "row_ln beta").data_ptr()
-        g.row_ln_counters = cnt.data_ptr(); g.row_ln_eps = eps
-        gemm_raw(g)
-        return out_f32, ln_out
     gemm_raw(g)
     return out_f32, out_bf16
-
-
-_ROW_LN_CNT = {}
-
-
-def _row_ln_counters(device, n: int) -> torch.Tensor:
-    """Arrival counters of the fused row LayerNorm (zero between launches: the kernel resets what it counts)."""
-    key = (device.type, device.index)
-    t = _ROW_LN_CNT.get(key)
-    if t is None or t.numel() < n:
-        t = torch.zeros((max(n, 4096),), dtype=I32, device=device)
-        _ROW_LN_CNT[key] = t
-    return t
 
 
 def split3_bf16(x: torch.Tensor, weight_layout: bool = False, scale: float = 1.0) -> torch.Tensor:
@@ -192,7 +162,7 @@ def conv_igemm(x: torch.Tensor, w: torch.Tensor, bias: Optional[torch.Tensor], k
     g = GemmArgs()
     g.a = x.data_ptr(); g.a_row_stride = Cc; g.a_seg_stride = T_in * Cc; g.a_rows = T_in; g.a_cols = Cc
     g.P = stride; g.taps = k; g.kb_per_tap = Cc // 64; g.a_col_per_nblk = 0
-    g.w = w.data_ptr(); g.N = N; g.block_n = CONV_LN_BLOCK_N if ln_gamma is not None else 0
+    g.w = w.data_ptr(); g.N = N; g.block_n = 0
     g.segs = B; g.rows_per_seg = T_out
     g.bias = _ptr(bias)
     g.gamma = _ptr(ln_gamma); g.beta = _ptr(ln_beta); g.residual = None
@@ -245,9 +215,6 @@ def posconv(x_pad: torch.Tensor, w: torch.Tensor, bias: Optional[torch.Tensor], 
     return out_f32
 
 
-# fused-LayerNorm conv tile: 0 / 256 = half-split (two 256-column accumulator halves, epilogue under the MMAs),
-# 512 = full-width tile (MMA and epilogue alternate); A/B runs
-CONV_LN_BLOCK_N = int(os.environ.get("APTAI_CONV_LN_BLOCK_N", "0"))
 CONV0_TC = int(os.environ.get("APTAI_CONV0_TC", "1"))     # 0: the SIMT conv-0 kernel (A/B runs)
 
 
@@ -321,12 +288,9 @@ def posconv_fold(g: torch.Tensor, v: torch.Tensor, cpad: int = 64, out: Optional
     return w
 
 
-SERPENTINE = int(os.environ.get("APTAI_SERPENTINE", "1"))         # 0: every kernel walks its rows front to back (A/B runs)
-
-
 def set_traversal(reverse: bool) -> None:
     """Traversal hint for the next GEMM / LayerNorm / attention-v3 launches of this thread (include/aptai_b200.h)."""
-    _lib.load().aptai_set_traversal(1 if (reverse and SERPENTINE) else 0)
+    _lib.load().aptai_set_traversal(1 if reverse else 0)
 
 
 class Serpentine:
@@ -343,24 +307,16 @@ class Serpentine:
         set_traversal(False)
 
 
-# 1: the LayerNorm behind out-proj / FFN2 of the pre-LN encoder runs inside those GEMM launches (linear(row_ln=...));
-# 0 (default): standalone LayerNorm launches.  Measured slower (bench 23.4 k -> 18.1 k audio-s/s, profiles/
-# row_ln_bench.py): the in-kernel normalisation starves behind the operand stream; kept as a tested experiment
-FUSED_ROW_LN = int(os.environ.get("APTAI_FUSED_ROW_LN", "0"))
-# 1: out-proj / FFN2 bias gradients come out of the LayerNorm backward that produces their dy (layernorm_bwd dcolsum);
-# 0: separate colsum launches (A/B runs)
-FUSED_BIAS_COLSUM = int(os.environ.get("APTAI_FUSED_BIAS_COLSUM", "1"))
 POSCONV_SLAB = int(os.environ.get("APTAI_POSCONV_SLAB", "1"))     # 0: always the generic implicit-GEMM path (A/B runs)
-
-# 0: by shape (attention_v3.cu's query-tile pairs with P in TMEM when an utterance has more than one 128-query tile,
-# else attention_tc.cu's two threads per row), 1 / 2 / 3: force one kernel (A/B runs in profiles/attn_bench.py)
-ATTENTION_IMPL = int(os.environ.get("APTAI_ATTN_IMPL", "0"))
-ATTENTION_POLY8 = int(os.environ.get("APTAI_ATTN_POLY8", "3"))
 
 
 def attention(qkv: torch.Tensor, key_len: Optional[torch.Tensor], B: int, T: int, heads: int,
               out: Optional[torch.Tensor] = None, lse: Optional[torch.Tensor] = None,
               impl: Optional[int] = None, drop_p: float = 0.0, drop_seed: int = 0) -> torch.Tensor:
+    """impl None: the kernel by shape (attention_v3.cu's query-tile pairs with P in TMEM when an utterance has more
+    than one 128-query tile, else attention_tc.cu's two threads per row); 1 / 3 force one of them (tests)."""
+    if impl not in (None, 1, 3):
+        raise ValueError(f"attention: impl must be None, 1 or 3, not {impl!r}")
     fmt = _h16(qkv, "qkv")
     H = heads * 64
     assert qkv.numel() == B * T * 3 * H
@@ -380,18 +336,14 @@ def attention(qkv: torch.Tensor, key_len: Optional[torch.Tensor], B: int, T: int
                                                       T, heads, float(drop_p), int(drop_seed) & 0xFFFFFFFFFFFFFFFF,
                                                       _stream()), "attention_fwd_dropout")
         return out
-    which = impl or ATTENTION_IMPL or (3 if T > 128 else 1)
+    which = impl or (3 if T > 128 else 1)
     if which == 3:
         check(_lib.load().aptai_attention_fwd_v3(qkv.data_ptr(), out.data_ptr(), _ptr(lse), key_len.data_ptr(), B, T,
-                                                 heads, ATTENTION_POLY8 | (fmt << 24), _stream()), "attention_fwd_v3")
+                                                 heads, fmt, _stream()), "attention_fwd_v3")
         return out
     if fmt:               # fp16 operands: the two-threads-per-row kernel for short utterances
         check(_lib.load().aptai_attention_fwd_fmt(qkv.data_ptr(), out.data_ptr(), _ptr(lse), key_len.data_ptr(), B, T,
                                                   heads, fmt, _stream()), "attention_fwd_fmt")
-        return out
-    if which == 2:
-        check(_lib.load().aptai_attention_fwd_v2(qkv.data_ptr(), out.data_ptr(), _ptr(lse), key_len.data_ptr(), B, T,
-                                                 heads, _stream()), "attention_fwd_v2")
         return out
     if lse is not None:
         check(_lib.load().aptai_attention_fwd_lse(qkv.data_ptr(), out.data_ptr(), lse.data_ptr(), key_len.data_ptr(),

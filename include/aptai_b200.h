@@ -61,8 +61,8 @@ typedef struct aptai_gemm_args {
   int32_t a_col_per_nblk; /* channel offset per n tile (grouped conv), else 0 */
   const void* w;          /* bf16 [N][K] */
   int32_t N;
-  int32_t block_n;        /* 0 = choose; otherwise one of 48, 64, 128, 256.  ln=1: 0 / 256 = half-split row tile (two
-                             256-column accumulator halves, epilogue overlapped with the MMAs), 512 = full-width tile */
+  int32_t block_n;        /* 0 = choose; otherwise one of 48, 64, 128, 256.  ln=1: 0 or 256, the half-split row tile
+                             (two 256-column accumulator halves, epilogue overlapped with the MMAs) */
   int32_t segs;
   int32_t rows_per_seg;   /* output rows per segment */
   const float* bias;      /* [N] or NULL */
@@ -83,16 +83,6 @@ typedef struct aptai_gemm_args {
   const void* aux;        /* act=2 only: bf16, same row mapping/ldo as the outputs: out = acc * gelu'(aux)  (dgrad of
                              HF:566-573 through the activation) */
   void* out_pre;          /* optional 16-bit copy of the value before the activation (kept for the backward pass) */
-  /* Fused LayerNorm of the UPDATED rows behind an in-place residual update (out_f32 == residual, nothing else
-   * written, act 0; N = 768 or 1024, one segment, ldo == N): row_ln_out[r][:] = LN(out_f32[r][:]) in the 16-bit format
-   * of half_fmt (pre-LN encoder, HF:639-655: the LayerNorm that follows out-proj / FFN2).  The CTA that completes a
-   * 128-row block's last column tile normalises the block out of L2.  row_ln_counters: int32, one per 128-row block
-   * (>= ceil(rows/256)*2 entries), all zero on entry; the launch leaves them zero.  NULL row_ln_out: off. */
-  void* row_ln_out;
-  const float* row_ln_gamma;   /* [N] */
-  const float* row_ln_beta;    /* [N] */
-  int32_t* row_ln_counters;
-  float row_ln_eps;
 } aptai_gemm_args;
 
 int aptai_gemm_bf16(const aptai_gemm_args* args, void* stream);
@@ -157,16 +147,11 @@ int aptai_attention_fwd(const void* qkv, void* ctx, const int32_t* key_len, int 
  * probabilities and the context carry three more mantissa bits at the same tensor-core rate); lse may be NULL */
 int aptai_attention_fwd_fmt(const void* qkv, void* ctx, float* lse, const int32_t* key_len, int B, int T, int heads,
                             int half_fmt, void* stream);
-/* second-generation tcgen05 kernel, same contract (+ optional lse, may be NULL): two 128-query tiles per CTA share one
- * K/V stream and run independent softmax chains (csrc/attention_tc2.cu) */
-int aptai_attention_fwd_v2(const void* qkv, void* ctx, float* lse, const int32_t* key_len, int B, int T, int heads,
-                           void* stream);
 /* third-generation kernel, same contract (csrc/attention_v3.cu): P stays in TMEM as the A operand of P V, three S
- * buffers per query tile, part of the exponentials on the FMA pipe, TMA store of the context tile.
- * poly8 bits 0..7: exponential pairs per 8 evaluated by the polynomial (0, 2, 3, 4; any other value selects the default
- * 3); bits 8..23: issuer back-off in ns (profiling); bit 24: qkv / ctx are IEEE fp16 instead of bf16. */
+ * buffers per query tile, 3 of every 8 exponential pairs on the FMA pipe, TMA store of the context tile.
+ * half_fmt as in aptai_attention_fwd_fmt (0 = bf16, 1 = IEEE fp16); lse may be NULL. */
 int aptai_attention_fwd_v3(const void* qkv, void* ctx, float* lse, const int32_t* key_len, int B, int T, int heads,
-                           int poly8, void* stream);
+                           int half_fmt, void* stream);
 
 /* ------------------------------------------------------------------ heads and post-processing ---------------
  * APTAI heads (models/aptai.py:43-55,83-86,105-106): tv = tanh(h) W_tv^T + b_tv (9), logits = leaky_relu(h)

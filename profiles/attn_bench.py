@@ -1,4 +1,5 @@
-"""Attention micro-benchmark: tcgen05 kernel vs the legacy mma.sync kernel (CUDA events, L2 flushed)."""
+"""Attention micro-benchmark: the by-shape default against the two-threads-per-row kernel (impl 1) and the
+query-tile-pair kernel with P in TMEM (impl 3) (CUDA events, L2 flushed)."""
 import os, sys
 import torch
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
@@ -21,13 +22,8 @@ for B, T in [(120, 399), (48, 999), (80, 600), (189, 250)]:
     kl = torch.full((B,), T, dtype=torch.int32, device=dev)
     out = torch.empty((B * T, H), dtype=torch.bfloat16, device=dev)
     fl = 4.0 * B * heads * T * T * 64
+    r = timeit(lambda: ops.attention(qkv, kl, B, T, heads, out=out))
     a = timeit(lambda: ops.attention(qkv, kl, B, T, heads, out=out, impl=1))
-    c = timeit(lambda: ops.attention(qkv, kl, B, T, heads, out=out, impl=2))
-    line = (f"B={B:4d} T={T:4d}: tcgen05 v1 {a:7.3f} ms {fl / a / 1e9:7.1f} TFLOP/s | v2 (q-tile pairs) {c:7.3f} ms "
-            f"{fl / c / 1e9:7.1f} TFLOP/s | v3 (P in TMEM), polynomial pairs per 8:")
-    for poly in (0, 2, 3, 4):
-        ops.ATTENTION_POLY8 = poly
-        d = timeit(lambda: ops.attention(qkv, kl, B, T, heads, out=out, impl=3))
-        line += f" [{poly & 255}] {d:7.3f} ms {fl / d / 1e9:7.1f}"
-    ops.ATTENTION_POLY8 = 3
-    print(line, flush=True)
+    d = timeit(lambda: ops.attention(qkv, kl, B, T, heads, out=out, impl=3))
+    print(f"B={B:4d} T={T:4d}: default {r:7.3f} ms {fl / r / 1e9:7.1f} TFLOP/s | impl 1 {a:7.3f} ms "
+          f"{fl / a / 1e9:7.1f} TFLOP/s | impl 3 (P in TMEM) {d:7.3f} ms {fl / d / 1e9:7.1f} TFLOP/s", flush=True)

@@ -6,7 +6,7 @@ kernels, tail, low-pass, log-softmax, CTC-Viterbi) in the three precision modes,
 import os, sys
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.dirname(os.path.abspath(__file__)))))
 import torch
-from aptai_b200 import APTAI, ops
+from aptai_b200 import APTAI
 from aptai_b200.backbone import register_in_memory_checkpoint
 from aptai_b200.config import W2V2Config
 from aptai_b200.synth import backbone_state_dict, waveforms
@@ -28,9 +28,3 @@ for mode in ("bf16", "fp16", "f32x3"):
     r1 = m.predict(wav[2:3, :16000].contiguous(), torch.tensor([16000], device=dev))
     torch.cuda.synchronize()
     print(mode, "ok", float(r["tvs_pred"].abs().max()), r["align_status"].tolist(), r1["phn_fc_logits"].shape, flush=True)
-# the opt-in fused row LayerNorm
-a = torch.randn((700, 1024), device=dev).bfloat16(); w = (torch.randn((1024, 1024), device=dev) * 0.02).bfloat16()
-h = torch.randn((700, 1024), device=dev); g = torch.ones((1024,), device=dev); b = torch.zeros((1024,), device=dev)
-ops.linear(a, w, b, residual=h, out_f32=h, want_bf16=False, row_ln=(g, b, 1e-5))
-torch.cuda.synchronize()
-print("row_ln ok", flush=True)

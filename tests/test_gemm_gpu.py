@@ -192,36 +192,3 @@ def test_linear_fp16_operands(cuda):
     h0 = h.clone()
     ops.linear(u, w2.half(), b2, residual=h, out_f32=h, want_bf16=False)
     torch.testing.assert_close(h, h0 + u.float() @ w2.half().float().t() + b2, atol=2e-4, rtol=2e-4)
-
-
-@pytest.mark.parametrize("M,K,N,dt", [(700, 1024, 1024, torch.bfloat16), (47880, 1024, 1024, torch.bfloat16),
-                                      (20000, 4096, 1024, torch.float16), (1000, 3072, 768, torch.bfloat16),
-                                      (1, 1024, 1024, torch.bfloat16), (75776, 1024, 1024, torch.float16)])
-def test_linear_row_ln(cuda, M, K, N, dt):
-    """In-place residual update + LayerNorm of the updated rows in ONE launch (row_ln): the CTA that lands a 128-row
-    block's last column tile normalises the block out of L2.  Same reduce-add update as the plain launch (bit for bit),
-    same LayerNorm arithmetic as the standalone kernel; counters return to zero; both traversal directions; single-CTA
-    and CTA-pair tiles (M = 700 / 1000 / 1 run 128-row tiles)."""
-    a = (_rand((M, K), cuda, 1.0, 70)).to(dt)
-    w = (_rand((N, K), cuda, 0.03, 71)).to(dt)
-    b = _rand((N,), cuda, 0.1, 72)
-    g = 1 + _rand((N,), cuda, 0.1, 73)
-    e = _rand((N,), cuda, 0.1, 74)
-    h0 = _rand((M, N), cuda, 1.0, 75)
-    h_ref = h0.clone()
-    ops.linear(a, w, b, residual=h_ref, out_f32=h_ref, want_bf16=False)
-    _, x_ref = ops.layernorm(h_ref, g, e, 1e-5, out16_dtype=dt)
-    for rev in (False, True, False):
-        h = h0.clone()
-        ops.set_traversal(rev)
-        try:
-            _, x = ops.linear(a, w, b, residual=h, out_f32=h, want_bf16=False, row_ln=(g, e, 1e-5))
-        finally:
-            ops.set_traversal(False)
-        assert x.dtype == dt and x.shape == (M, N)
-        assert torch.equal(h, h_ref)
-        torch.testing.assert_close(x.float(), x_ref.float(), atol=1e-2, rtol=1e-2)
-        assert float((x != x_ref).float().mean()) < 1e-3          # the same arithmetic: at most stray 1-ulp differences
-        assert int(ops._row_ln_counters(cuda, 1).abs().sum()) == 0
-    with pytest.raises(ValueError):
-        ops.linear(a, w, b, want_f32=True, want_bf16=False, row_ln=(g, e, 1e-5))

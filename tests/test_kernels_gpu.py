@@ -95,7 +95,7 @@ def test_layernorm(cuda, cols, in_bf16):
     torch.testing.assert_close(o16.float(), ref.bfloat16().float(), atol=2e-2, rtol=1e-2)
 
 
-@pytest.mark.parametrize("legacy", [False, "v2", "v3", "v3p0", "v3p4"])
+@pytest.mark.parametrize("legacy", [False, "v3"])
 @pytest.mark.parametrize("B,T,heads,lens,scale", [(2, 199, 16, [199, 150], 1.0), (3, 64, 12, [64, 1, 33], 1.0),
                                                   (1, 999, 4, [999], 1.0), (2, 130, 2, [70, 130], 1.0),
                                                   (40, 399, 16, None, 0.5), (2, 513, 2, [513, 400], 3.0),
@@ -110,20 +110,12 @@ def test_attention(cuda, B, T, heads, lens, scale, legacy):
         qkv[T // 2:, H: 2 * H] *= 4.0          # later keys score much higher: exercises the lazy O rescale
     kl = torch.tensor(lens, dtype=torch.int32, device=cuda)
     lse = None
-    if legacy == "v2":
+    if legacy == "v3":
+        # third generation (P in TMEM, polynomial exponentials for 3 of every 8 pairs); context buffer pre-filled so
+        # that rows the TMA store must NOT touch (none here: every row < T is written) would show
         lse = torch.empty((B, heads, T), dtype=torch.float32, device=cuda)
-        ctx = ops.attention(qkv, kl, B, T, heads, impl=2, lse=lse)
-    elif legacy in ("v3", "v3p0", "v3p4"):
-        # third generation (P in TMEM, polynomial exponentials for 3 / 0 / 4 of every 8 pairs); context buffer
-        # pre-filled so that rows the TMA store must NOT touch (none here: every row < T is written) would show
-        lse = torch.empty((B, heads, T), dtype=torch.float32, device=cuda)
-        old = ops.ATTENTION_POLY8
-        ops.ATTENTION_POLY8 = {"v3": 3, "v3p0": 0, "v3p4": 4}[legacy]
-        try:
-            ctx = ops.attention(qkv, kl, B, T, heads, impl=3, lse=lse,
-                                out=torch.full((B * T, H), float("nan"), dtype=torch.bfloat16, device=cuda))
-        finally:
-            ops.ATTENTION_POLY8 = old
+        ctx = ops.attention(qkv, kl, B, T, heads, impl=3, lse=lse,
+                            out=torch.full((B * T, H), float("nan"), dtype=torch.bfloat16, device=cuda))
     else:
         ctx = ops.attention(qkv, kl, B, T, heads, impl=1)
     q, k, v = qkv.float().view(B, T, 3, heads, 64).permute(2, 0, 3, 1, 4)
